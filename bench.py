@@ -2,7 +2,17 @@
 """Headline benchmark: train samples/sec of the Swin-V2 + T5 image-caption step (BASELINE.json `metric`).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference|hf_eager] [--workload 2a|3|4a|5|2b|1a|tiny] [--batch B]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
+
+--dump-outputs DIR writes what the last timed step of our arm computed as DIR/<name>.npy (float32 / float64), so that two builds
+run with the same arguments can be compared output for output (inputs, weights and dropout masks are seeded):
+  training workloads: loss.npy (the loss the step read back) and transformer_params.npy (a fixed seeded sample of 2^20
+                      elements of the transformer weights after the step's Adam update)
+  decode workload 5:  generated_ids.npy (the greedy ids of the last generate() call, as float64)
+Two runs agree only as far as the step is deterministic: the shared-embedding and T5 relative-bias gradients are summed with
+floating-point atomics whose order varies from run to run, and over several bf16 training steps those last-bit differences
+in the weights spread to every later gradient and weight update.
 
 A "step" is exactly what /root/reference/train.py:54-71 does per batch with accumulation_steps = 1:
     (host->device copy of the batch) -> loss = model(images, src, tgt) -> loss.item() -> loss.backward() ->
@@ -35,6 +45,7 @@ from __future__ import annotations
 import argparse
 import json
 import os
+import random
 import subprocess
 import sys
 import threading
@@ -538,6 +549,39 @@ def _gemm_traffic_from_profiles():
         return json.load(fh)
 
 
+DUMP_SAMPLE = 1 << 20
+DUMP_MAX_BYTES = 64 << 20
+
+
+def _flat_sample(tensors, n, seed):
+    """A fixed, seeded sample of n elements (drawn with replacement, in index order) of `tensors` taken as one flat vector, as
+    float32 on the host; every element when they hold no more than n."""
+    import numpy as np
+    sizes = [t.numel() for t in tensors]
+    total = sum(sizes)
+    if total <= n:
+        return torch.cat([t.detach().reshape(-1).float().cpu() for t in tensors]).numpy()
+    idx = torch.randint(total, (n,), generator=torch.Generator().manual_seed(seed)).sort().values
+    out, off, lo = [], 0, 0
+    for t, s in zip(tensors, sizes):
+        hi = int(torch.searchsorted(idx, off + s))
+        if hi > lo:
+            out.append(t.detach().reshape(-1)[(idx[lo:hi] - off).to(t.device)].float().cpu())
+        off, lo = off + s, hi
+    return np.concatenate([o.numpy() for o in out])
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each array as out_dir/<name>.npy (float32 / float64 only, DUMP_MAX_BYTES in all)."""
+    import numpy as np
+    assert all(a.dtype in (np.float32, np.float64) for a in arrays.values())
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+    print(f"[bench] wrote {', '.join(f'{k}.npy {tuple(a.shape)}' for k, a in arrays.items())} to {out_dir}", file=sys.stderr)
+
+
 def _timed_steps(fn, k, flush, world, dev):
     """Time EXACTLY k steps as ONE region: barrier + synchronize, start event, k x (L2 flush, step), wait for every side stream the
     steps left work on (the fused Adam runs on its own stream and overlaps the NEXT step's towers), end event, synchronize; max over
@@ -691,6 +735,8 @@ def run_decode(args, w):
         l0 = O.launch_count() + POOL.replayed_kernels
         ms_res, ids = _timed_steps(resident, args.steps, flush, 1, dev)
         launches = O.launch_count() + POOL.replayed_kernels - l0
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"generated_ids": ids.cpu().double().numpy()})
         hi = sampler.mark()
         for _ in range(max(args.warmup, 3)):
             e2e()
@@ -852,6 +898,10 @@ def run_ours(args, w):
     l0 = O.launch_count() + POOL.replayed_kernels
     ms_res, loss_v = _timed_steps(resident_step, args.steps, flush, world, dev)
     launches = O.launch_count() + POOL.replayed_kernels - l0
+    if args.dump_outputs and rank == 0:                  # before any further step changes the weights
+        import numpy as np
+        dump_outputs(args.dump_outputs, {"loss": np.array([loss_v], dtype=np.float64),
+                                         "transformer_params": _flat_sample(list(model.transformer.parameters()), DUMP_SAMPLE, 1)})
     ms_iso = _timed_steps_isolated(resident_step, args.steps, flush, dev) if world == 1 else None
     hi = sampler.mark() if sampler else 0
     for _ in range(max(args.warmup, 3)):                 # the e2e path allocates its device batches on the prefetch stream: let the
@@ -980,7 +1030,10 @@ def main():
     ap.add_argument("--profile-range", action="store_true",
                     help="for ncu --profile-from-start off: cudaProfilerStart/Stop around the K steps after warm-up, then exit (no JSON line)")
     ap.add_argument("--gemm-probe", action="store_true", help="development aid: only replay (and check) the step's GEMM signatures")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    random.seed(0)                                 # the dropout counter starts from Python's `random` (modeling.step_seed)
     global _REAL_STDOUT
     sys.stdout.flush()
     _REAL_STDOUT = os.dup(1)

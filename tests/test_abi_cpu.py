@@ -88,16 +88,28 @@ def test_state_dict_layout_matches_reference_keys():
 
 
 def test_state_dict_layout_matches_transformers_if_present():
-    transformers = pytest.importorskip("transformers")
+    """Against the layout transformers 5.5.0 stored in tests/golden/hf_layout.json (tests/golden/make_hf_golden.py), and
+    against the installed transformers classes where they import."""
+    import json
+
     from klab_multimodalmodel_b200.modeling import Swinv2Config, Swinv2Model, T5Config, T5ForConditionalGeneration
+    from tests.golden.make_hf_golden import LAYOUT_SWIN, LAYOUT_T5
+    ours = T5ForConditionalGeneration(T5Config(**LAYOUT_T5))
+    sw = Swinv2Model(Swinv2Config(**LAYOUT_SWIN, pretrained_window_sizes=(0, 0, 0)))
+    with open(os.path.join(ROOT, "tests", "golden", "hf_layout.json")) as fh:
+        stored = json.load(fh)
+    for model, layout in ((ours, stored["t5"]), (sw, stored["swin"])):
+        assert set(layout) == set(model.state_dict())
+        model.load_state_dict({k: torch.zeros(shape) for k, shape in layout.items()}, strict=True)
+    try:
+        import transformers
+    except ImportError:
+        return
     hf = transformers.T5ForConditionalGeneration(transformers.T5Config(vocab_size=512, d_model=128, d_kv=64, d_ff=256, num_layers=2,
                                                                        num_heads=2, decoder_start_token_id=0))
-    ours = T5ForConditionalGeneration(T5Config(vocab_size=512, d_model=128, d_ff=256, num_layers=2, num_heads=2))
     assert set(hf.state_dict()) == set(ours.state_dict())
     ours.load_state_dict(hf.state_dict(), strict=True)
     hfs = transformers.Swinv2Model(transformers.Swinv2Config(image_size=64, embed_dim=32, depths=[2, 2, 2], num_heads=[1, 2, 4], window_size=4))
-    sw = Swinv2Model(Swinv2Config(image_size=64, embed_dim=32, depths=(2, 2, 2), num_heads=(1, 2, 4), window_size=4,
-                                  pretrained_window_sizes=(0, 0, 0)))
     assert set(hfs.state_dict()) == set(sw.state_dict())
     sw.load_state_dict(hfs.state_dict(), strict=True)
 
