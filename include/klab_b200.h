@@ -160,6 +160,20 @@ int klab_t5_attention_bwd(void* stream, int dtype, int B, int H, int Lq, int Lk,
                           int rel_zero, int num_buckets, int causal, int q_offset, const float* lse, float* dbias_table,
                           float dropout_p, unsigned long long seed, const unsigned long long* seed_ptr, void* workspace);
 long long klab_t5_attention_bwd_workspace_bytes(int B, int H, int Lq, int num_buckets);
+/* Beam-search decode attention (one query row per hypothesis; the rows of one sample are consecutive).  Same arithmetic as the
+ * Lq = 1 forward above, except where keys come from:
+ *   src != NULL (self-attention): key / value position j of query row r is cache row src[r * ld_src + j] * Lk + j of k / v
+ *     (Lk = cache positions per hypothesis); causal bound j <= q_offset; T5 bias as above.  src is the beam ancestry table of
+ *     klab_beam_update: it replaces HF's per-step cache reorder (HF/generation/utils.py:3330-3336).
+ *   src == NULL (cross-attention): the kv_group consecutive query rows r of one sample share its K/V rows
+ *     [(r / kv_group) * Lk, ... + Lk) -- the encoder output is projected once per sample, not per beam
+ *     (HF's _expand_inputs_for_generation repeats it).  No bias, no mask.
+ * kv_group query rows (1..32) run in one CTA and consume each K/V chunk from shared memory.  bf16 (16-byte loads) or fp32 (the
+ * exact path); fp32 arithmetic either way. */
+int klab_t5_attention_decode_beam(void* stream, int dtype, int rows, int H, int Lk, int d_kv, const void* q, long long ldq,
+                                  const void* k, long long ldk, const void* v, long long ldv, void* out, long long ldo,
+                                  int kv_group, const int* src, long long ld_src, const float* bias_table, const int* rel_bucket,
+                                  int rel_zero, int q_offset);
 
 /* ---- K2+K3+K4: Swin-V2 shifted-window cosine attention (HF/models/swinv2/modeling_swinv2.py:421-487,
  * window_partition/roll/reverse :146-166,:678,:698, shift mask :627-653) -------------------------------
@@ -227,6 +241,23 @@ int klab_lmhead_ce_bwd_chunk(void* stream, long long rows, int d, const void* h,
  * unfinished[b] &= ids[b,t] != eos.  logits are fp32 [B,V]; ties resolve to the lowest index. */
 int klab_greedy_step(void* stream, int B, int V, const float* logits, long long ld, long long* ids, long long ld_ids, int t,
                      int* unfinished, int pad_id, int eos_id);
+
+/* ---- K14 (part): beam search step on device state (HF/generation/utils.py:3076-3386, GenerationMixin._beam_search of 5.5.0,
+ * one EOS id so k = 2 * num_beams candidates are kept).  Ties resolve to the lower flat index beam * V + token.
+ * klab_beam_topk: per row of the fp32 logits [rows, V]: log_softmax (fp32) + run_scores[row], its k largest values, descending,
+ *   as cand_val [rows, k] and token ids cand_tok [rows, k].  k even, 4..16.
+ * klab_beam_update: one step for the token at position t + 1 of B samples of nb (2..8) running beams (rows b * nb + i):
+ *   merges the nb * 2nb candidates, applies EOS / max-length (T new tokens), chooses the next running beams (run_scores,
+ *   next_tok [B * nb] int64), merges the finished set (fin_scores: score / generated_len ** length_penalty, fin_seq, fin_flag,
+ *   fin_len), updates the early-stop heuristic (unsat [B]) and done [B] (early_stopping 0 False, 1 True, 2 "never").
+ *   src (int32), run_seq and fin_seq (int64) are double-buffered [2][B * nb][ld], ld >= T + 1: buffer t & 1 is read and
+ *   (t + 1) & 1 written; src[r, j] is the cache row that holds position j of hypothesis r.  A sample with done[b] set no longer
+ *   changes (its tables are carried forward unchanged); unsat and done must start at 1 and 0. */
+int klab_beam_topk(void* stream, int rows, int V, int k, const float* logits, long long ld, const float* run_scores, float* cand_val,
+                   int* cand_tok);
+int klab_beam_update(void* stream, int B, int nb, int V, int T, int t, int eos_id, float length_penalty, int early_stopping,
+                     const float* cand_val, const int* cand_tok, float* run_scores, int* src, long long* run_seq, long long ld,
+                     float* fin_scores, long long* fin_seq, int* fin_flag, int* fin_len, int* unsat, int* done, long long* next_tok);
 
 /* y = x * keep(seed, linear index)/(1-p): the mask klab_gemm's epilogue dropout applied to a contiguous [M,N] output
  * (T5 dropout sites, HF/models/t5/modeling_t5.py:95,149,375,406,734,768), regenerated for the backward pass. */

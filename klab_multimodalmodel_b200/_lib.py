@@ -73,6 +73,7 @@ SIGNATURES = {
     "klab_t5_attention_bwd": [_vp, _i, _i, _i, _i, _i, _i, _vp, _ll, _vp, _ll, _vp, _ll, _vp, _vp, _ll, _vp, _vp, _vp, _vp, _vp,
                               _i, _i, _i, _i, _vp, _vp, _f, _ull, _vp, _vp],
     "klab_t5_attention_bwd_workspace_bytes": [_i, _i, _i, _i],
+    "klab_t5_attention_decode_beam": [_vp, _i, _i, _i, _i, _i, _vp, _ll, _vp, _ll, _vp, _ll, _vp, _ll, _i, _vp, _ll, _vp, _vp, _i, _i],
     "klab_swin_attention_fwd": [_vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _ll, _vp, _ll, _vp, _vp, _vp],
     "klab_swin_attention_bwd": [_vp, _i, _i, _i, _i, _i, _i, _i, _vp, _vp, _vp, _ll, _vp, _vp, _ll, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "klab_swin_cpb_fwd": [_vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
@@ -89,6 +90,8 @@ SIGNATURES = {
     "klab_lmhead_ce_bwd_chunk": [_vp, _ll, _i, _vp, _ll, _vp, _ll, _f, _vp, _vp, _vp, _vp, _i, _i, _vp, _ll],
     "klab_cast": [_vp, _i, _i, _ll, _vp, _vp],
     "klab_greedy_step": [_vp, _i, _i, _vp, _ll, _vp, _ll, _i, _vp, _i, _i],
+    "klab_beam_topk": [_vp, _i, _i, _i, _vp, _ll, _vp, _vp, _vp],
+    "klab_beam_update": [_vp, _i, _i, _i, _i, _i, _i, _f, _i, _vp, _vp, _vp, _vp, _vp, _ll, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "klab_dropout_apply": [_vp, _i, _ll, _vp, _vp, _f, _ull, _vp],
     "klab_seed_advance": [_vp, _vp],
     "klab_adam_chunk_elems": [],

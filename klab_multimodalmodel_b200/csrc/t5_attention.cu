@@ -427,6 +427,117 @@ int set_smem(K kern, size_t bytes) {
     return KLAB_OK;
 }
 
+// ------------------------------------------------------------------------------------------------------------------
+// Beam-search decode attention (klab_t5_attention_decode_beam): one query row per hypothesis, the nb hypotheses of one sample
+// in consecutive rows.  One CTA per (sample, head) with one warp per beam; keys are streamed in chunks of CK through shared
+// memory (fp32), online softmax per warp, fp32 arithmetic throughout (expf / fmaf: the fp32 variant is the exact path).
+//   self-attention (src != null): key position j of row r lives in cache row src[r, j] * Lk + j -- the ancestry table replaces
+//     HF's per-step cache reorder (cache.reorder_cache) -- with the causal bound j <= q_offset and the T5 relative bias;
+//   cross-attention (src == null): all kv_group rows of a sample read that sample's [Lk, .] K/V, so each chunk is fetched once
+//     per CTA and consumed by every beam: the cross K/V stream of a step does not grow with the number of beams.
+// ------------------------------------------------------------------------------------------------------------------
+struct BeamAttnArgs {
+    const void *q, *k, *v;
+    void* out;
+    long long ldq, ldk, ldv, ldo;
+    int G, H, Lk, dk;                 // G = rows per CTA (beams of a sample)
+    const int* src;                   // [rows, ld_src] or null
+    long long ld_src;
+    const float* bias_table;
+    const int* rel_bucket;
+    int rel_zero, q_offset;
+};
+
+__device__ __forceinline__ void load_vec_f32(const __nv_bfloat16* p, float* dst) {      // 8 elements, one 16-byte load
+    float f[8];
+    unpack8_bf16(__ldg(reinterpret_cast<const uint4*>(p)), f);
+#pragma unroll
+    for (int i = 0; i < 8; ++i) dst[i] = f[i];
+}
+__device__ __forceinline__ void load_vec_f32(const float* p, float* dst) { dst[0] = __ldg(p); }
+
+template <typename T, bool SELF, int CK>
+__global__ void t5_attn_decode_beam_kernel(BeamAttnArgs a) {
+    extern __shared__ float sm[];
+    const int dk = a.dk, dp = dk + 1, G = a.G;
+    constexpr int VEC = sizeof(T) == 2 ? 8 : 1;               // elements per load
+    const int regions = SELF ? G : 1;
+    float* Ks = sm;                                           // [regions][CK][dp]
+    float* Vs = Ks + regions * CK * dp;
+    float* qs = Vs + regions * CK * dp;                       // [G][dk]
+    const int grp = blockIdx.x, h = blockIdx.y;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const int row = grp * G + warp;
+    const T* qp = reinterpret_cast<const T*>(a.q) + static_cast<long long>(row) * a.ldq + h * dk;
+    for (int c = lane; c < dk; c += 32) qs[warp * dk + c] = to_f32(qp[c]);
+    const int jmax = SELF ? min(a.Lk, a.q_offset + 1) : a.Lk;
+    const int nthr = blockDim.x;
+    const int per_row = dk / VEC;
+    float m = -INFINITY, l = 0.0f;
+    float acc[4] = {0.f, 0.f, 0.f, 0.f};                      // columns lane + 32 i (d_kv <= 128)
+    const float* Kw = Ks + (SELF ? warp : 0) * CK * dp;
+    const float* Vw = Vs + (SELF ? warp : 0) * CK * dp;
+    for (int j0 = 0; j0 < jmax; j0 += CK) {
+        __syncthreads();                                      // previous chunk consumed
+        for (int e = threadIdx.x; e < regions * CK * per_row; e += nthr) {
+            const int g = e / (CK * per_row), rem = e % (CK * per_row), jj = rem / per_row, c = (rem % per_row) * VEC;
+            const int j = j0 + jj;
+            if (j >= jmax) continue;
+            long long krow;
+            if (SELF) krow = static_cast<long long>(__ldg(a.src + static_cast<long long>(grp * G + g) * a.ld_src + j)) * a.Lk + j;
+            else krow = static_cast<long long>(grp) * a.Lk + j;
+            const T* kp = reinterpret_cast<const T*>(a.k) + krow * a.ldk + h * dk + c;
+            const T* vp = reinterpret_cast<const T*>(a.v) + krow * a.ldv + h * dk + c;
+            float* kd = Ks + (g * CK + jj) * dp + c;
+            float* vd = Vs + (g * CK + jj) * dp + c;
+            load_vec_f32(kp, kd);
+            load_vec_f32(vp, vd);
+        }
+        __syncthreads();
+        const int j = j0 + lane;
+        float sc = -INFINITY;
+        if (lane < CK && j < jmax) {
+            const float* kr = Kw + lane * dp;
+            const float* qw = qs + warp * dk;
+            float t = 0.0f;
+            for (int c = 0; c < dk; ++c) t = fmaf(qw[c], kr[c], t);
+            if (SELF && a.bias_table) t += __ldg(a.bias_table + __ldg(a.rel_bucket + (j - a.q_offset) + a.rel_zero) * a.H + h);
+            sc = t;
+        }
+        const float m_new = fmaxf(m, warp_max(sc));                // finite: every chunk holds a visible key
+        const float corr = expf(m - m_new);
+        const float p = expf(sc - m_new);                          // masked lanes: exp(-inf) = 0
+        l = l * corr + warp_sum(p);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) acc[i] *= corr;
+        const int nk = min(CK, jmax - j0);
+        for (int jj = 0; jj < nk; ++jj) {
+            const float pj = __shfl_sync(0xffffffffu, p, jj);
+            const float* vr = Vw + jj * dp;
+#pragma unroll
+            for (int i = 0; i < 4; ++i)
+                if (lane + 32 * i < dk) acc[i] = fmaf(pj, vr[lane + 32 * i], acc[i]);
+        }
+        m = m_new;
+    }
+    const float inv = 1.0f / l;
+    T* op = reinterpret_cast<T*>(a.out) + static_cast<long long>(row) * a.ldo + h * dk;
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+        if (lane + 32 * i < dk) op[lane + 32 * i] = from_f32<T>(acc[i] * inv);
+}
+
+template <typename T, bool SELF, int CK>
+int launch_decode_beam(cudaStream_t st, const BeamAttnArgs& a, int groups) {
+    const int regions = SELF ? a.G : 1;
+    const size_t smem = sizeof(float) * (2ull * regions * CK * (a.dk + 1) + 1ull * a.G * a.dk);
+    if (int rc = set_smem(t5_attn_decode_beam_kernel<T, SELF, CK>, smem)) return rc;
+    t5_attn_decode_beam_kernel<T, SELF, CK><<<dim3(groups, a.H), a.G * 32, smem, st>>>(a);
+    KLAB_LAUNCH_CHECK();
+    count_launch();
+    return KLAB_OK;
+}
+
 }  // namespace
 
 // tensor-core path (t5_attention_tc.cu)
@@ -499,6 +610,31 @@ int klab_t5_attention_fwd(void* stream, int dtype, int B, int H, int Lq, int Lk,
     KLAB_LAUNCH_CHECK();
     count_launch();
     return KLAB_OK;
+}
+
+int klab_t5_attention_decode_beam(void* stream, int dtype, int rows, int H, int Lk, int d_kv, const void* q, long long ldq,
+                                  const void* k, long long ldk, const void* v, long long ldv, void* out, long long ldo,
+                                  int kv_group, const int* src, long long ld_src, const float* bias_table, const int* rel_bucket,
+                                  int rel_zero, int q_offset) {
+    if (int rc = klab_check_device()) return rc;
+    KLAB_REQUIRE(rows > 0 && H > 0 && Lk > 0 && d_kv > 0 && d_kv <= 128 && kv_group >= 1 && kv_group <= 32 && rows % kv_group == 0,
+                 "t5_attention_decode_beam: bad shape rows=%d H=%d Lk=%d d_kv=%d kv_group=%d", rows, H, Lk, d_kv, kv_group);
+    KLAB_REQUIRE(!src || (q_offset >= 0 && q_offset < Lk && ld_src > q_offset), "t5_attention_decode_beam: q_offset %d outside the cache",
+                 q_offset);
+    if (dtype == KLAB_BF16)
+        KLAB_REQUIRE(d_kv % 8 == 0 && ((ldq | ldk | ldv) & 7) == 0 &&
+                     ((reinterpret_cast<uintptr_t>(k) | reinterpret_cast<uintptr_t>(v)) & 15) == 0,
+                     "t5_attention_decode_beam: bf16 K/V need d_kv and row strides multiple of 8 and 16-byte aligned bases");
+    BeamAttnArgs a{};
+    a.q = q; a.k = k; a.v = v; a.out = out;
+    a.ldq = ldq; a.ldk = ldk; a.ldv = ldv; a.ldo = ldo;
+    a.G = kv_group; a.H = H; a.Lk = Lk; a.dk = d_kv;
+    a.src = src; a.ld_src = ld_src; a.bias_table = bias_table; a.rel_bucket = rel_bucket; a.rel_zero = rel_zero; a.q_offset = q_offset;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int groups = rows / kv_group;
+    if (dtype == KLAB_BF16)
+        return src ? launch_decode_beam<__nv_bfloat16, true, 16>(st, a, groups) : launch_decode_beam<__nv_bfloat16, false, 32>(st, a, groups);
+    return src ? launch_decode_beam<float, true, 16>(st, a, groups) : launch_decode_beam<float, false, 32>(st, a, groups);
 }
 
 int klab_t5_attention_bwd(void* stream, int dtype, int B, int H, int Lq, int Lk, int d_kv, const void* q, long long ldq,

@@ -10,6 +10,7 @@ projected once before the loop.  Every step is one token per sample: O(T) work i
 The step for position t is a CUDA-graph region (graphs.py) over static buffers, so the launch-bound chain of small kernels
 costs one graph launch per token.
 `greedy_generate_recompute` is that older prefix-recompute schedule, kept as a cross-check (identical ids; tests).
+`beam_generate` is beam search (`generate(num_beams=k)`) on the same cached single-token step, see below.
 """
 from __future__ import annotations
 
@@ -165,3 +166,136 @@ def greedy_generate_recompute(tr, embeds, B, Le, max_new_tokens: int = 20):
         if not bool(unfinished.cpu().any()):                           # HF checks the stopping criteria every step too
             break
     return ids[:, :n_out]
+
+
+# ------------------------------------------------------------------------------------------------------------------------------
+# Beam search: GenerationMixin._beam_search of HF 5.5.0 (HF/generation/utils.py:3076-3386) on device state.  Rows are
+# hypotheses, b * nb + i.  Unlike HF, the encoder output is NOT repeated per beam (the cross-attention kernel lets the nb rows
+# of a sample share its K/V) and the self-attention cache is never reordered: row r writes its token-t keys / values into its
+# own cache row (r, t), and the ancestry table src[r, j] (klab_beam_update) says which row holds position j of hypothesis r.
+# ------------------------------------------------------------------------------------------------------------------------------
+_EARLY_STOPPING = {False: 0, True: 1, "never": 2}
+
+
+class _BeamState:
+    """Static device buffers of one beam-search geometry (B, nb, Le, T): everything the per-position graph regions read or write."""
+
+    def __init__(self, tr, B, nb, Le, T, cd, dev):
+        cfg = tr.config
+        inner = cfg.num_heads * cfg.d_kv
+        n = len(tr.decoder.block)
+        R = B * nb
+        self.enc = torch.empty(B * Le, cfg.d_model, dtype=cd, device=dev)
+        self.cross_kv = [torch.empty(B * Le, 2 * inner, dtype=cd, device=dev) for _ in range(n)]      # once per sample
+        self.self_qkv = [torch.zeros(R * T, 3 * inner, dtype=cd, device=dev) for _ in range(n)]      # row (r, t)
+        self.lut, self.rz = tr.decoder.lut(T, dev)
+        self.src = torch.empty(2, R, T + 1, dtype=torch.int32, device=dev)
+        self.run_seq = torch.empty(2, R, T + 1, dtype=torch.int64, device=dev)
+        self.fin_seq = torch.empty(2, R, T + 1, dtype=torch.int64, device=dev)
+        self.run_scores = torch.empty(R, dtype=torch.float32, device=dev)
+        self.fin_scores = torch.empty(R, dtype=torch.float32, device=dev)
+        self.fin_flag = torch.empty(R, dtype=torch.int32, device=dev)
+        self.fin_len = torch.empty(R, dtype=torch.int32, device=dev)
+        self.unsat = torch.empty(B, dtype=torch.int32, device=dev)
+        self.done = torch.empty(B, dtype=torch.int32, device=dev)
+        self.next_tok = torch.empty(R, 1, dtype=torch.int64, device=dev)
+        self.cand_val = torch.empty(R, 2 * nb, dtype=torch.float32, device=dev)
+        self.cand_tok = torch.empty(R, 2 * nb, dtype=torch.int32, device=dev)
+
+    def reset(self, cfg, nb):
+        """HF's initial state (:3185-3199); unused positions hold `pad_token_id or eos_token_id` (:3187), EOS for T5."""
+        fill = cfg.pad_token_id or cfg.eos_token_id
+        R = self.run_scores.shape[0]
+        self.src.copy_(torch.arange(R, dtype=torch.int32, device=self.src.device)[None, :, None].expand_as(self.src))
+        for s in (self.run_seq, self.fin_seq):
+            s.fill_(fill)
+            s[:, :, 0] = cfg.decoder_start_token_id
+        self.run_scores.view(-1, nb).fill_(-1e9)
+        self.run_scores.view(-1, nb)[:, 0] = 0.0
+        self.fin_scores.fill_(-1e9)
+        self.fin_flag.zero_()
+        self.fin_len.zero_()
+        self.unsat.fill_(1)
+        self.done.zero_()
+        self.next_tok.fill_(cfg.decoder_start_token_id)
+
+
+def _beam_step_body(tr, st, t, B, nb, Le, T, length_penalty, early_stopping):
+    """Position t for every hypothesis, then top-k and the beam update.  Reads and writes `st` and the operand cache only."""
+    cfg = tr.config
+    cd = st.enc.dtype
+    H, dk, d, eps = cfg.num_heads, cfg.d_kv, cfg.d_model, cfg.layer_norm_epsilon
+    inner = H * dk
+    R = B * nb
+    V = tr.shared.weight.shape[0]
+    layers, tab = _decode_operands_peek(tr, cd)
+    table = tr.decoder.block[0].layer[0].SelfAttention.relative_attention_bias.weight.detach()
+    src = st.src[t & 1]
+    x = O.embedding_fwd(st.next_tok, tab)                          # [R, d]
+    for l, (ln0, wqkv, w_o, ln1, w_cq, _w_ckv, w_co, ln2, w_i, w_ff) in enumerate(layers):
+        self_qkv, cross_kv = st.self_qkv[l], st.cross_kv[l]
+        n0, _ = O.rmsnorm_fwd(x, ln0, eps, save_stats=False)
+        row_t = self_qkv.view(R, T, 3 * inner)[:, t]
+        O.linear_fwd(n0, wqkv, out=row_t)
+        ctx = O.t5_attention_decode_beam(row_t[:, :inner], self_qkv[:, inner:2 * inner], self_qkv[:, 2 * inner:], R, H, T, dk,
+                                         kv_group=nb, src=src, bias_table=table, lut=st.lut, rel_zero=st.rz, q_offset=t)
+        h1 = O.linear_fwd(ctx, w_o, residual=x)
+        n1, _ = O.rmsnorm_fwd(h1, ln1, eps, save_stats=False)
+        qc = O.linear_fwd(n1, w_cq)
+        ctx2 = O.t5_attention_decode_beam(qc, cross_kv[:, :inner], cross_kv[:, inner:], R, H, Le, dk, kv_group=nb)
+        h2 = O.linear_fwd(ctx2, w_co, residual=h1)
+        n2, _ = O.rmsnorm_fwd(h2, ln2, eps, save_stats=False)
+        f = O.linear_fwd(n2, w_i, act=L.ACT_RELU)
+        x = O.linear_fwd(f, w_ff, residual=h2)
+    n, _ = O.rmsnorm_fwd(x, tr.decoder.final_layer_norm.weight, eps, save_stats=False)
+    logits = O.linear_fwd(n, tab, alpha=d ** -0.5, out_dtype=torch.float32)
+    lib, stream = L.lib(), torch.cuda.current_stream().cuda_stream
+    K = 2 * nb
+    L.check(lib.klab_beam_topk(stream, R, V, K, logits.data_ptr(), logits.stride(0), st.run_scores.data_ptr(), st.cand_val.data_ptr(),
+                               st.cand_tok.data_ptr()))
+    L.check(lib.klab_beam_update(stream, B, nb, V, T, t, cfg.eos_token_id, float(length_penalty), _EARLY_STOPPING[early_stopping],
+                                 st.cand_val.data_ptr(), st.cand_tok.data_ptr(), st.run_scores.data_ptr(), st.src.data_ptr(),
+                                 st.run_seq.data_ptr(), T + 1, st.fin_scores.data_ptr(), st.fin_seq.data_ptr(), st.fin_flag.data_ptr(),
+                                 st.fin_len.data_ptr(), st.unsat.data_ptr(), st.done.data_ptr(), st.next_tok.data_ptr()))
+    return (st.fin_scores,)
+
+
+@torch.no_grad()
+def beam_generate(tr, embeds, B, Le, num_beams: int, max_new_tokens: int = 20, length_penalty: float = 1.0, early_stopping=False,
+                  num_return_sequences: int = 1):
+    """-> (sequences [B * num_return_sequences, n] int64, sequences_scores [B * num_return_sequences] fp32), as
+    `generate(inputs_embeds, num_beams=...)` of HF 5.5.0 returns them (:3368-3376)."""
+    from .graphs import POOL
+    cfg = tr.config
+    cd = embeds.dtype
+    dev = embeds.device
+    nb, T = num_beams, max_new_tokens
+    states = tr.__dict__.setdefault("_klab_beam_states", {})
+    key = (B, nb, Le, T, cd, dev)
+    st = states.get(key)
+    if st is None:
+        if len(states) >= 4:                                             # as greedy_generate: a handful of geometries at most
+            dead = {id(o) for o in states.values()}
+            POOL.drop_keys(lambda k: k[0] == "beam" and k[2] in dead)
+            states.clear()
+        st = states[key] = _BeamState(tr, B, nb, Le, T, cd, dev)
+    enc = tr.encoder.run_blocks(embeds, B, Le, tr.cache)
+    O.rmsnorm_fwd(enc, tr.encoder.final_layer_norm.weight, cfg.layer_norm_epsilon, out=st.enc, save_stats=False)
+    layers, _ = _decode_operands(tr, cd)
+    for l, ops_l in enumerate(layers):
+        O.linear_fwd(st.enc, ops_l[5], out=st.cross_kv[l])
+    st.reset(cfg, nb)
+    # A sample whose finished set can no longer change is frozen on the device (klab_beam_update), so running past the step at
+    # which HF stops changes nothing: the "every sample done" flag is read back every CHECK_EVERY steps only.
+    n_run = 0
+    for t in range(T):
+        POOL.run(("beam", id(tr), id(st), t, float(length_penalty), _EARLY_STOPPING[early_stopping]), _beam_step_body, (),
+                 (tr, st, t, B, nb, Le, T, length_penalty, early_stopping))
+        n_run = t + 1
+        if n_run % CHECK_EVERY == 0 and n_run < T and bool(st.done.cpu().all()):
+            break
+    nrs = num_return_sequences
+    seq = st.fin_seq[n_run & 1].view(B, nb, T + 1)[:, :nrs].reshape(B * nrs, T + 1)
+    scores = st.fin_scores.view(B, nb)[:, :nrs].reshape(B * nrs).clone()
+    n_out = 1 + int(st.fin_len.view(B, nb)[:, :nrs].max().item())
+    return seq[:, :n_out].clone(), scores

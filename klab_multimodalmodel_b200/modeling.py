@@ -373,6 +373,35 @@ class T5EncoderModel(nn.Module):
         return self.encoder.run_blocks(x, B, L_, self.cache)
 
 
+class GenerationConfig:
+    """The `generation_config` fields of HF 5.5.0 (HF/generation/configuration_utils.py) that this build supports, with their
+    defaults; the token ids come from the model config.  Setting `num_beams` > 1 here makes `generate()` -- and so
+    `MyModel.forward(return_loss=False)` -- run beam search, as in the reference."""
+
+    def __init__(self, cfg: "T5Config"):
+        self.max_length = 20
+        self.max_new_tokens = None
+        self.num_beams = 1
+        self.length_penalty = 1.0
+        self.early_stopping = False
+        self.num_return_sequences = 1
+        self.decoder_start_token_id = cfg.decoder_start_token_id
+        self.eos_token_id = cfg.eos_token_id
+        self.pad_token_id = cfg.pad_token_id
+
+
+@dataclass
+class BeamSearchOutput:
+    """`generate(..., return_dict_in_generate=True, output_scores=True)`: sequences and, for beam search, the scores of the
+    returned hypotheses (None for greedy decoding)."""
+    sequences: torch.Tensor
+    sequences_scores: torch.Tensor | None = None
+
+
+_GEN_FIELDS = ("max_length", "max_new_tokens", "num_beams", "length_penalty", "early_stopping", "num_return_sequences")
+_MAX_BEAMS = 8
+
+
 class T5ForConditionalGeneration(nn.Module):
     """Trainable encoder-decoder of the reference (/root/reference/models/model.py:17,26,28)."""
 
@@ -385,6 +414,7 @@ class T5ForConditionalGeneration(nn.Module):
         self.lm_head = _P(cfg.vocab_size, cfg.d_model)
         self.lm_head.weight = self.shared.weight                     # tied (HF/models/t5/modeling_t5.py:956-960)
         self.cache = OperandCache()
+        self.generation_config = GenerationConfig(cfg)
         init_t5_(self)
 
     @classmethod
@@ -424,6 +454,47 @@ class T5ForConditionalGeneration(nn.Module):
         dec = self.decoder.run_blocks(dec_in, B, Lt, self.cache, enc_out=enc, Le=Le)
         return Fn.apply_fn(Fn.LMHeadLossFn, dec, self.decoder.final_layer_norm.weight, self.shared.weight, labels, self.cache,
                            cfg.layer_norm_epsilon, p, self.decoder.seed_base + 7, sp)
+
+    def generate(self, inputs_embeds=None, return_dict_in_generate=False, output_scores=False, **overrides):
+        """`generate(inputs_embeds=[B, Le, d], **overrides)` of HF 5.5.0 for the options in `generation_config`: greedy decoding
+        (num_beams 1) or beam search (num_beams 2..8).  The compute dtype is that of inputs_embeds (bf16 or fp32).  Returns the
+        ids [B * num_return_sequences, n] int64, or with return_dict_in_generate=True a BeamSearchOutput (sequences_scores needs
+        output_scores=True).  Options this build does not implement raise instead of being ignored."""
+        from . import generation
+        unknown = sorted(set(overrides) - set(_GEN_FIELDS))
+        if unknown:
+            raise ValueError(f"generate(): {', '.join(unknown)} not supported (supported: {', '.join(_GEN_FIELDS)}, "
+                             "return_dict_in_generate, output_scores); sampling and logits processors are not implemented")
+        gc = self.generation_config
+        opt = {k: overrides.get(k, getattr(gc, k)) for k in _GEN_FIELDS}
+        nb, nrs, es = opt["num_beams"], opt["num_return_sequences"], opt["early_stopping"]
+        if not isinstance(nb, int) or not 1 <= nb <= _MAX_BEAMS:
+            raise ValueError(f"generate(): num_beams={nb!r}; this build supports 1..{_MAX_BEAMS}")
+        if not isinstance(nrs, int) or not 1 <= nrs <= nb:
+            raise ValueError(f"generate(): num_return_sequences={nrs!r} must be in 1..num_beams ({nb})")
+        if es not in (False, True, "never") or isinstance(es, int) and not isinstance(es, bool):
+            raise ValueError(f"generate(): early_stopping={es!r} must be False, True or 'never'")
+        # HF/generation/utils.py:1608-1640 (_prepare_generated_length) for an encoder-decoder whose decoder prompt is the start token
+        if opt["max_new_tokens"] is not None:
+            T = int(opt["max_new_tokens"])
+        elif "max_length" in overrides or gc.max_length != 20:
+            T = int(opt["max_length"]) - 1
+        else:
+            T = 20
+        if T < 1:
+            raise ValueError(f"generate(): nothing to generate (max_new_tokens {T})")
+        if inputs_embeds is None or inputs_embeds.dim() != 3:
+            raise ValueError("generate(): inputs_embeds [B, Le, d_model] is required")
+        B, Le, d = inputs_embeds.shape
+        x = inputs_embeds.reshape(B * Le, d)
+        if nb == 1:
+            seqs, scores = generation.greedy_generate(self, x, B, Le, max_new_tokens=T), None
+        else:
+            seqs, scores = generation.beam_generate(self, x, B, Le, num_beams=nb, max_new_tokens=T, length_penalty=float(opt["length_penalty"]),
+                                                    early_stopping=es, num_return_sequences=nrs)
+        if return_dict_in_generate:
+            return BeamSearchOutput(seqs, scores if output_scores else None)
+        return seqs
 
 
 def init_t5_(m: nn.Module, seed: int | None = None):

@@ -24,7 +24,6 @@ import torch.distributed as dist
 from torch import nn
 
 from .. import functional as Fn
-from ..generation import greedy_generate
 from ..graphs import POOL
 from ..modeling import Swinv2Model, T5EncoderModel, T5ForConditionalGeneration, _compute_dtype, advance_step_seed
 from ..optim import allow_overlap, wait_pending_updates
@@ -115,8 +114,8 @@ class MyModel(nn.Module):
         if return_loss:
             return self.transformer.loss_from_embeds(emb, B, Le, target_encoding["input_ids"])
         else:
-            with torch.no_grad():
-                return greedy_generate(self.transformer, emb, B, Le)
+            with torch.no_grad():               # model.py:28 of the reference: greedy unless generation_config says otherwise
+                return self.transformer.generate(inputs_embeds=emb.view(B, Le, emb.shape[-1]))
 
     def save(self, result_name="best.pth"):
         result_path = os.path.join(self.args.result_dir, result_name)

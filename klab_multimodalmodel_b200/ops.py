@@ -250,6 +250,18 @@ def t5_attention_fwd(q, k, v, B, H, Lq, Lk, dk, *, bias_table=None, lut=None, re
     return ctx, lse
 
 
+def t5_attention_decode_beam(q, k, v, rows, H, Lk, dk, *, kv_group, src=None, bias_table=None, lut=None, rel_zero=0, q_offset=0,
+                             out=None):
+    """One query row per hypothesis: self-attention through the ancestry table `src` [rows, ld] int32, or (src None)
+    cross-attention where `kv_group` consecutive rows share one sample's Lk K/V rows."""
+    ctx = torch.empty(rows, H * dk, dtype=q.dtype, device=q.device) if out is None else out
+    L.check(L.lib().klab_t5_attention_decode_beam(_stream(), _DT[q.dtype], rows, H, Lk, dk, q.data_ptr(), q.stride(0), k.data_ptr(),
+                                                  k.stride(0), v.data_ptr(), v.stride(0), ctx.data_ptr(), ctx.stride(0), kv_group,
+                                                  _p(src), 0 if src is None else src.stride(0), _p(bias_table), _p(lut), rel_zero,
+                                                  q_offset))
+    return ctx
+
+
 def t5_attention_bwd(q, k, v, ctx, dctx, lse, dq, dk_, dv, B, H, Lq, Lk, dk, *, bias_table=None, lut=None, rel_zero=0,
                      num_buckets=32, causal=False, q_offset=0, dbias_table=None, dropout_p=0.0, seed=0, seed_ptr=None):
     """dq / dk_ / dv are preallocated outputs with the same row strides as q / k / v."""
