@@ -242,6 +242,20 @@ int klab_lmhead_ce_bwd_chunk(void* stream, long long rows, int d, const void* h,
 int klab_greedy_step(void* stream, int B, int V, const float* logits, long long ld, long long* ids, long long ld_ids, int t,
                      int* unfinished, int pad_id, int eos_id);
 
+/* ---- K14 (part): multinomial sampling step (HF/generation/utils.py:2658-2800 with do_sample=True): per row of the fp32
+ * logits [rows, V], unfinished rows draw ids[row, t] from softmax(warped logits), finished rows get pad_id;
+ * unfinished[row] &= ids[row, t] != eos.  Warpers in HF's order: logits / temperature; top_k > 0 keeps scores >= the k-th
+ * largest (ties kept; top_k >= V keeps all); top_p < 1 keeps token i iff the mass of the tokens with a strictly greater score
+ * is < top_p, or i holds the maximum (ties at the boundary are all kept; top_p = 0 keeps the maximum and its ties).
+ * The draw: u = u(*seed, row, t - 1) -- t - 1 is the number of tokens generated before this one -- with
+ *   z = seed + 0x9E3779B97F4A7C15 * (1 + row * 2^16 + (t - 1)) mod 2^64, the splitmix64 finaliser on z, u = (z >> 40) * 2^-24;
+ * the token is the smallest index i with sum_{j <= i, kept} exp(s_j - max) > u * Z, Z the sum over the kept tokens (the last
+ * kept token if rounding leaves none).  seed is a DEVICE pointer (read at run time, so a captured graph draws anew when the
+ * value there changes).  The row is held in shared memory: V too large for it returns an error.  t in 1..65536. */
+int klab_sample_step(void* stream, int rows, int V, const float* logits, long long ld, long long* ids, long long ld_ids, int t,
+                     int* unfinished, int pad_id, int eos_id, float temperature, int top_k, float top_p,
+                     const unsigned long long* seed);
+
 /* ---- K14 (part): beam search step on device state (HF/generation/utils.py:3076-3386, GenerationMixin._beam_search of 5.5.0,
  * one EOS id so k = 2 * num_beams candidates are kept).  Ties resolve to the lower flat index beam * V + token.
  * klab_beam_topk: per row of the fp32 logits [rows, V]: log_softmax (fp32) + run_scores[row], its k largest values, descending,

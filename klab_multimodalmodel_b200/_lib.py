@@ -90,6 +90,7 @@ SIGNATURES = {
     "klab_lmhead_ce_bwd_chunk": [_vp, _ll, _i, _vp, _ll, _vp, _ll, _f, _vp, _vp, _vp, _vp, _i, _i, _vp, _ll],
     "klab_cast": [_vp, _i, _i, _ll, _vp, _vp],
     "klab_greedy_step": [_vp, _i, _i, _vp, _ll, _vp, _ll, _i, _vp, _i, _i],
+    "klab_sample_step": [_vp, _i, _i, _vp, _ll, _vp, _ll, _i, _vp, _i, _i, _f, _i, _f, _vp],
     "klab_beam_topk": [_vp, _i, _i, _i, _vp, _ll, _vp, _vp, _vp],
     "klab_beam_update": [_vp, _i, _i, _i, _i, _i, _i, _f, _i, _vp, _vp, _vp, _vp, _vp, _ll, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "klab_dropout_apply": [_vp, _i, _ll, _vp, _vp, _f, _ull, _vp],

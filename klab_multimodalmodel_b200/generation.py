@@ -11,6 +11,8 @@ The step for position t is a CUDA-graph region (graphs.py) over static buffers, 
 costs one graph launch per token.
 `greedy_generate_recompute` is that older prefix-recompute schedule, kept as a cross-check (identical ids; tests).
 `beam_generate` is beam search (`generate(num_beams=k)`) on the same cached single-token step, see below.
+`sample_generate` is multinomial sampling (`generate(do_sample=True)`): greedy's state, loop and step with klab_sample_step in
+place of the argmax, see below.
 """
 from __future__ import annotations
 
@@ -25,16 +27,18 @@ class _DecodeState:
     self-attention q|k|v cache and the cross-attention k|v projection.  They never move, so the kernel sequence of the
     single-token step for position t can be captured into a CUDA graph once and replayed for every later caption batch."""
 
-    def __init__(self, tr, B, Le, T, cd, dev):
+    def __init__(self, tr, B, Le, T, cd, dev, rows=None):
         cfg = tr.config
         inner = cfg.num_heads * cfg.d_kv
         n = len(tr.decoder.block)
-        self.ids = torch.empty(B, T + 1, dtype=torch.int64, device=dev)
-        self.tok = torch.empty(B, 1, dtype=torch.int64, device=dev)
-        self.unfinished = torch.empty(B, dtype=torch.int32, device=dev)
+        R = B if rows is None else rows                            # decoded rows: B, or B * num_return_sequences when sampling
+        self.ids = torch.empty(R, T + 1, dtype=torch.int64, device=dev)
+        self.tok = torch.empty(R, 1, dtype=torch.int64, device=dev)
+        self.unfinished = torch.empty(R, dtype=torch.int32, device=dev)
+        self.seed = torch.zeros(1, dtype=torch.int64, device=dev)  # sampling: the call's seed, read by the kernel at run time
         self.enc = torch.empty(B * Le, cfg.d_model, dtype=cd, device=dev)
-        self.cross_kv = [torch.empty(B * Le, 2 * inner, dtype=cd, device=dev) for _ in range(n)]
-        self.self_qkv = [torch.zeros(B * T, 3 * inner, dtype=cd, device=dev) for _ in range(n)]   # row (b, t): q | k | v of token t
+        self.cross_kv = [torch.empty(B * Le, 2 * inner, dtype=cd, device=dev) for _ in range(n)]   # once per sample
+        self.self_qkv = [torch.zeros(R * T, 3 * inner, dtype=cd, device=dev) for _ in range(n)]   # row (r, t): q | k | v of token t
         self.lut, self.rz = tr.decoder.lut(T, dev)                 # covers relative positions -(T-1) .. T-1
 
 
@@ -48,38 +52,50 @@ def _decode_operands(tr, cd):
     return out, g([tr.shared.weight], cd)
 
 
-def _decode_step_body(tr, st, t, B, Le, T):
-    """One token for every sample: position t in, ids[:, t + 1] out.  consts only (no per-call inputs): everything it reads or
-    writes lives in `st` or in the operand cache, so the region is capturable as is."""
+def _decode_step_body(tr, st, t, B, Le, T, sample=None):
+    """One token for every row: position t in, ids[:, t + 1] out.  consts only (no per-call inputs): everything it reads or
+    writes lives in `st` or in the operand cache, so the region is capturable as is.  sample None: greedy (B rows, argmax);
+    sample = (n, temperature, top_k, top_p): B * n rows drawn by klab_sample_step, the n rows of a sample sharing its
+    cross-attention K/V."""
     cfg = tr.config
+    n_rs = 1 if sample is None else sample[0]
+    R = B * n_rs
     cd = st.enc.dtype
     H, dk, d, eps = cfg.num_heads, cfg.d_kv, cfg.d_model, cfg.layer_norm_epsilon
     inner = H * dk
     layers, tab = _decode_operands_peek(tr, cd)
     table = tr.decoder.block[0].layer[0].SelfAttention.relative_attention_bias.weight.detach()
     st.tok.copy_(st.ids[:, t:t + 1])
-    x = O.embedding_fwd(st.tok, tab)                               # [B, d]
+    x = O.embedding_fwd(st.tok, tab)                               # [R, d]
     for l, (ln0, wqkv, w_o, ln1, w_cq, _w_ckv, w_co, ln2, w_i, w_ff) in enumerate(layers):
         self_qkv, cross_kv = st.self_qkv[l], st.cross_kv[l]
         n0, _ = O.rmsnorm_fwd(x, ln0, eps, save_stats=False)
-        row_t = self_qkv.view(B, T, 3 * inner)[:, t]               # [B, 3*inner] view, row stride T*3*inner
+        row_t = self_qkv.view(R, T, 3 * inner)[:, t]               # [R, 3*inner] view, row stride T*3*inner
         O.linear_fwd(n0, wqkv, out=row_t)                          # q | k | v of the new token, written into the cache
-        ctx, _ = O.t5_attention_fwd(row_t[:, :inner], self_qkv[:, inner:2 * inner], self_qkv[:, 2 * inner:], B, H, 1, T, dk,
+        ctx, _ = O.t5_attention_fwd(row_t[:, :inner], self_qkv[:, inner:2 * inner], self_qkv[:, 2 * inner:], R, H, 1, T, dk,
                                     bias_table=table, lut=st.lut, rel_zero=st.rz, num_buckets=cfg.relative_attention_num_buckets,
                                     causal=True, q_offset=t)
         h1 = O.linear_fwd(ctx, w_o, residual=x)
         n1, _ = O.rmsnorm_fwd(h1, ln1, eps, save_stats=False)
         qc = O.linear_fwd(n1, w_cq)
-        ctx2, _ = O.t5_attention_fwd(qc, cross_kv[:, :inner], cross_kv[:, inner:], B, H, 1, Le, dk)
+        if n_rs == 1:
+            ctx2, _ = O.t5_attention_fwd(qc, cross_kv[:, :inner], cross_kv[:, inner:], B, H, 1, Le, dk)
+        else:                                                      # the n rows of a sample read its K/V (no per-row copy)
+            ctx2 = O.t5_attention_decode_beam(qc, cross_kv[:, :inner], cross_kv[:, inner:], R, H, Le, dk, kv_group=n_rs)
         h2 = O.linear_fwd(ctx2, w_co, residual=h1)
         n2, _ = O.rmsnorm_fwd(h2, ln2, eps, save_stats=False)
         f = O.linear_fwd(n2, w_i, act=L.ACT_RELU)
         x = O.linear_fwd(f, w_ff, residual=h2)
     n, _ = O.rmsnorm_fwd(x, tr.decoder.final_layer_norm.weight, eps, save_stats=False)
     logits = O.linear_fwd(n, tab, alpha=d ** -0.5, out_dtype=torch.float32)
-    L.check(L.lib().klab_greedy_step(torch.cuda.current_stream().cuda_stream, B, tr.shared.weight.shape[0], logits.data_ptr(),
-                                     logits.stride(0), st.ids.data_ptr(), st.ids.stride(0), t + 1, st.unfinished.data_ptr(),
-                                     cfg.pad_token_id, cfg.eos_token_id))
+    if sample is None:
+        L.check(L.lib().klab_greedy_step(torch.cuda.current_stream().cuda_stream, B, tr.shared.weight.shape[0], logits.data_ptr(),
+                                         logits.stride(0), st.ids.data_ptr(), st.ids.stride(0), t + 1, st.unfinished.data_ptr(),
+                                         cfg.pad_token_id, cfg.eos_token_id))
+    else:
+        _, temperature, top_k, top_p = sample
+        O.sample_step(logits, st.ids, t + 1, st.unfinished, st.seed, pad_id=cfg.pad_token_id, eos_id=cfg.eos_token_id,
+                      temperature=temperature, top_k=top_k, top_p=top_p)
     return (st.ids,)
 
 
@@ -96,22 +112,25 @@ def _decode_operands_peek(tr, cd):
 CHECK_EVERY = 5           # decode steps between two read-backs of the "every row has finished" flag
 
 
-@torch.no_grad()
-def greedy_generate(tr, embeds, B, Le, max_new_tokens: int = 20):
+def _decode_state(tr, attr, tag, key, make):
+    """The static state of one decode geometry, kept on the model in tr.__dict__[attr]; regions are keyed (tag, id(tr), id(st), ...)."""
     from .graphs import POOL
-    cfg = tr.config
-    cd = embeds.dtype
-    dev = embeds.device
-    T = max_new_tokens                                                   # decoder positions 0 .. T-1 are ever attended to
-    states = tr.__dict__.setdefault("_klab_decode_states", {})
-    key = (B, Le, T, cd, dev)
+    states = tr.__dict__.setdefault(attr, {})
     st = states.get(key)
     if st is None:
         if len(states) >= 4:                                             # a handful of geometries at most: the caches are large
             dead = {id(o) for o in states.values()}                      # the per-position regions bake the old buffers in: drop
-            POOL.drop_keys(lambda k: k[0] == "dec" and k[2] in dead)     # them too, or the states would never be freed
+            POOL.drop_keys(lambda k: k[0] == tag and k[2] in dead)       # them too, or the states would never be freed
             states.clear()
-        st = states[key] = _DecodeState(tr, B, Le, T, cd, dev)
+        st = states[key] = make()
+    return st
+
+
+def _decode_run(tr, st, embeds, B, Le, T, key, sample=None):
+    """Encoder, cross K|V and the cached single-token loop over the rows of `st`; -> ids [rows, n] cropped where HF stops."""
+    from .graphs import POOL
+    cfg = tr.config
+    cd = embeds.dtype
     enc = tr.encoder.run_blocks(embeds, B, Le, tr.cache)
     O.rmsnorm_fwd(enc, tr.encoder.final_layer_norm.weight, cfg.layer_norm_epsilon, out=st.enc, save_stats=False)
     layers, _ = _decode_operands(tr, cd)                                 # also validates / refreshes every operand copy
@@ -127,16 +146,25 @@ def greedy_generate(tr, embeds, B, Le, max_new_tokens: int = 20):
     for t in range(T):
         # the single-token step is ~11 small kernels per block: launch bound when issued one by one, so it is a captured region
         # per position t (keys beyond t are masked by the causal bound, stale cache rows of an earlier batch never contribute)
-        POOL.run(("dec", id(tr), id(st), t), _decode_step_body, (), (tr, st, t, B, Le, T))
+        POOL.run(key + (t,), _decode_step_body, (), (tr, st, t, B, Le, T) + ((sample,) if sample is not None else ()))
         n_run = t + 1
         if n_run % CHECK_EVERY == 0 and n_run < T and not bool(st.unfinished.cpu().any()):
             break
     ids = st.ids[:, :n_run + 1]
     # length HF would have returned: it stops right after the step in which the last unfinished row emitted EOS
     is_eos = ids[:, 1:] == cfg.eos_token_id
-    first_eos = torch.where(is_eos.any(1), is_eos.int().argmax(1) + 1, torch.full((B,), n_run, device=dev))     # tokens a row emits
+    first_eos = torch.where(is_eos.any(1), is_eos.int().argmax(1) + 1, torch.full((ids.shape[0],), n_run, device=ids.device))
     n_out = 1 + int(first_eos.max().item())
     return ids[:, :n_out].clone()
+
+
+@torch.no_grad()
+def greedy_generate(tr, embeds, B, Le, max_new_tokens: int = 20):
+    cd = embeds.dtype
+    dev = embeds.device
+    T = max_new_tokens                                                   # decoder positions 0 .. T-1 are ever attended to
+    st = _decode_state(tr, "_klab_decode_states", "dec", (B, Le, T, cd, dev), lambda: _DecodeState(tr, B, Le, T, cd, dev))
+    return _decode_run(tr, st, embeds, B, Le, T, ("dec", id(tr), id(st)))
 
 
 @torch.no_grad()
@@ -299,3 +327,53 @@ def beam_generate(tr, embeds, B, Le, num_beams: int, max_new_tokens: int = 20, l
     scores = st.fin_scores.view(B, nb)[:, :nrs].reshape(B * nrs).clone()
     n_out = 1 + int(st.fin_len.view(B, nb)[:, :nrs].max().item())
     return seq[:, :n_out].clone(), scores
+
+
+# ------------------------------------------------------------------------------------------------------------------------------
+# Multinomial sampling: GenerationMixin._sample of HF 5.5.0 (HF/generation/utils.py:2658-2800) with do_sample=True and the
+# temperature / top-k / top-p warpers, on the greedy machinery above.  num_return_sequences n expands sample b into the rows
+# b * n + j as HF does, but the encoder output is not repeated: the n rows share the sample's cross K/V.  The draw is
+# klab_sample_step's: a function of (seed, row, tokens generated so far) only, the seed one 63-bit number per call from torch's
+# default CPU generator, so torch.manual_seed makes a call reproducible, whether graphs are on or off.
+# ------------------------------------------------------------------------------------------------------------------------------
+MAX_RETURN_SEQUENCES = 32          # rows of one sample that share its K/V in one CTA of klab_t5_attention_decode_beam
+
+
+def check_sampling_options(temperature, top_k, top_p, num_return_sequences):
+    """ValueError for options outside what transformers accepts (GenerationConfig.validate) or this build supports."""
+    if isinstance(temperature, bool) or not isinstance(temperature, (int, float)) or not temperature > 0 or temperature == float("inf"):
+        raise ValueError(f"sampling: temperature={temperature!r} must be a positive number")
+    if isinstance(top_k, bool) or not isinstance(top_k, int) or top_k < 0:
+        raise ValueError(f"sampling: top_k={top_k!r} must be a non-negative int (0 disables it)")
+    if isinstance(top_p, bool) or not isinstance(top_p, (int, float)) or not 0.0 <= top_p <= 1.0:
+        raise ValueError(f"sampling: top_p={top_p!r} must be in [0, 1]")
+    n = num_return_sequences
+    if isinstance(n, bool) or not isinstance(n, int) or not 1 <= n <= MAX_RETURN_SEQUENCES:
+        raise ValueError(f"sampling: num_return_sequences={n!r} must be in 1..{MAX_RETURN_SEQUENCES}")
+
+
+def draw_seed() -> int:
+    """The seed of one sampling call: a 63-bit number from torch's default CPU generator (torch.manual_seed reproduces it)."""
+    return int(torch.randint(0, 2 ** 63 - 1, (), dtype=torch.int64))
+
+
+@torch.no_grad()
+def sample_generate(tr, embeds, B, Le, max_new_tokens: int = 20, temperature: float = 1.0, top_k: int = 50, top_p: float = 1.0,
+                    num_return_sequences: int = 1):
+    """`generate(inputs_embeds, do_sample=True, ...)` -> ids [B * num_return_sequences, n] int64 (rows b * n + j), embeds
+    [B * Le, d_model] bf16 or fp32 on the GPU."""
+    cfg = tr.config
+    if not (torch.is_tensor(embeds) and embeds.is_cuda and embeds.dtype in (torch.bfloat16, torch.float32) and embeds.dim() == 2
+            and embeds.shape == (B * Le, cfg.d_model)):
+        desc = f"{tuple(embeds.shape)} {embeds.dtype} on {embeds.device}" if torch.is_tensor(embeds) else type(embeds).__name__
+        raise ValueError(f"sample_generate: inputs_embeds must be a CUDA bf16 / fp32 tensor [B * Le, {cfg.d_model}] (got {desc})")
+    check_sampling_options(temperature, top_k, top_p, num_return_sequences)
+    cd = embeds.dtype
+    dev = embeds.device
+    n, T = num_return_sequences, max_new_tokens
+    seed = draw_seed()
+    st = _decode_state(tr, "_klab_sample_states", "samp", (B, n, Le, T, cd, dev),
+                       lambda: _DecodeState(tr, B, Le, T, cd, dev, rows=B * n))
+    st.seed.copy_(torch.tensor([seed], dtype=torch.int64))
+    sample = (n, float(temperature), int(top_k), float(top_p))
+    return _decode_run(tr, st, embeds, B, Le, T, ("samp", id(tr), id(st)) + sample, sample)

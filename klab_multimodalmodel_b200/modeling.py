@@ -376,7 +376,8 @@ class T5EncoderModel(nn.Module):
 class GenerationConfig:
     """The `generation_config` fields of HF 5.5.0 (HF/generation/configuration_utils.py) that this build supports, with their
     defaults; the token ids come from the model config.  Setting `num_beams` > 1 here makes `generate()` -- and so
-    `MyModel.forward(return_loss=False)` -- run beam search, as in the reference."""
+    `MyModel.forward(return_loss=False)` -- run beam search, as in the reference; setting `do_sample = True` makes it sample.
+    The sampling defaults are those HF applies when do_sample is set (configuration_utils.py:559-561)."""
 
     def __init__(self, cfg: "T5Config"):
         self.max_length = 20
@@ -385,6 +386,10 @@ class GenerationConfig:
         self.length_penalty = 1.0
         self.early_stopping = False
         self.num_return_sequences = 1
+        self.do_sample = False
+        self.temperature = 1.0
+        self.top_k = 50
+        self.top_p = 1.0
         self.decoder_start_token_id = cfg.decoder_start_token_id
         self.eos_token_id = cfg.eos_token_id
         self.pad_token_id = cfg.pad_token_id
@@ -398,7 +403,9 @@ class BeamSearchOutput:
     sequences_scores: torch.Tensor | None = None
 
 
-_GEN_FIELDS = ("max_length", "max_new_tokens", "num_beams", "length_penalty", "early_stopping", "num_return_sequences")
+_GEN_FIELDS = ("max_length", "max_new_tokens", "num_beams", "length_penalty", "early_stopping", "num_return_sequences", "do_sample",
+               "temperature", "top_k", "top_p")
+_SAMPLING_DEFAULTS = {"temperature": 1.0, "top_k": 50, "top_p": 1.0}
 _MAX_BEAMS = 8
 
 
@@ -457,21 +464,34 @@ class T5ForConditionalGeneration(nn.Module):
 
     def generate(self, inputs_embeds=None, return_dict_in_generate=False, output_scores=False, **overrides):
         """`generate(inputs_embeds=[B, Le, d], **overrides)` of HF 5.5.0 for the options in `generation_config`: greedy decoding
-        (num_beams 1) or beam search (num_beams 2..8).  The compute dtype is that of inputs_embeds (bf16 or fp32).  Returns the
-        ids [B * num_return_sequences, n] int64, or with return_dict_in_generate=True a BeamSearchOutput (sequences_scores needs
-        output_scores=True).  Options this build does not implement raise instead of being ignored."""
+        (num_beams 1), beam search (num_beams 2..8) or multinomial sampling (do_sample=True, num_beams 1, with temperature, top_k
+        and top_p).  The compute dtype is that of inputs_embeds (bf16 or fp32).  Returns the ids [B * num_return_sequences, n]
+        int64, or with return_dict_in_generate=True a BeamSearchOutput (sequences_scores needs output_scores=True and beam
+        search).  Options this build does not implement raise instead of being ignored."""
         from . import generation
         unknown = sorted(set(overrides) - set(_GEN_FIELDS))
         if unknown:
             raise ValueError(f"generate(): {', '.join(unknown)} not supported (supported: {', '.join(_GEN_FIELDS)}, "
-                             "return_dict_in_generate, output_scores); sampling and logits processors are not implemented")
+                             "return_dict_in_generate, output_scores); logits processors are not implemented")
         gc = self.generation_config
         opt = {k: overrides.get(k, getattr(gc, k)) for k in _GEN_FIELDS}
-        nb, nrs, es = opt["num_beams"], opt["num_return_sequences"], opt["early_stopping"]
+        nb, nrs, es, sample = opt["num_beams"], opt["num_return_sequences"], opt["early_stopping"], opt["do_sample"]
         if not isinstance(nb, int) or not 1 <= nb <= _MAX_BEAMS:
             raise ValueError(f"generate(): num_beams={nb!r}; this build supports 1..{_MAX_BEAMS}")
-        if not isinstance(nrs, int) or not 1 <= nrs <= nb:
-            raise ValueError(f"generate(): num_return_sequences={nrs!r} must be in 1..num_beams ({nb})")
+        if not isinstance(sample, bool):
+            raise ValueError(f"generate(): do_sample={sample!r} must be True or False")
+        if sample:
+            if nb > 1:
+                raise ValueError("generate(): do_sample=True with num_beams > 1 (beam sampling) is not implemented")
+            generation.check_sampling_options(opt["temperature"], opt["top_k"], opt["top_p"], nrs)
+        else:
+            # GenerationConfig.validate(strict=True) (HF/generation/configuration_utils.py:636-660): flags that only matter when
+            # sampling.  transformers warns and ignores them; ignoring an option silently is what this build never does
+            flags = [f"{k}={opt[k]!r}" for k, v in _SAMPLING_DEFAULTS.items() if opt[k] != v]
+            if flags:
+                raise ValueError(f"generate(): {', '.join(flags)} only apply when sampling: set do_sample=True")
+            if not isinstance(nrs, int) or not 1 <= nrs <= nb:
+                raise ValueError(f"generate(): num_return_sequences={nrs!r} must be in 1..num_beams ({nb})")
         if es not in (False, True, "never") or isinstance(es, int) and not isinstance(es, bool):
             raise ValueError(f"generate(): early_stopping={es!r} must be False, True or 'never'")
         # HF/generation/utils.py:1608-1640 (_prepare_generated_length) for an encoder-decoder whose decoder prompt is the start token
@@ -487,7 +507,10 @@ class T5ForConditionalGeneration(nn.Module):
             raise ValueError("generate(): inputs_embeds [B, Le, d_model] is required")
         B, Le, d = inputs_embeds.shape
         x = inputs_embeds.reshape(B * Le, d)
-        if nb == 1:
+        if sample:
+            seqs, scores = generation.sample_generate(self, x, B, Le, max_new_tokens=T, temperature=opt["temperature"],
+                                                      top_k=opt["top_k"], top_p=opt["top_p"], num_return_sequences=nrs), None
+        elif nb == 1:
             seqs, scores = generation.greedy_generate(self, x, B, Le, max_new_tokens=T), None
         else:
             seqs, scores = generation.beam_generate(self, x, B, Le, num_beams=nb, max_new_tokens=T, length_penalty=float(opt["length_penalty"]),

@@ -262,6 +262,14 @@ def t5_attention_decode_beam(q, k, v, rows, H, Lk, dk, *, kv_group, src=None, bi
     return ctx
 
 
+def sample_step(logits, ids, t, unfinished, seed, *, pad_id, eos_id, temperature=1.0, top_k=0, top_p=1.0):
+    """Draw ids[:, t] from the warped fp32 logits [rows, V] (klab_sample_step); seed is a one-element int64 device tensor."""
+    rows, V = logits.shape
+    L.check(L.lib().klab_sample_step(_stream(), rows, V, logits.data_ptr(), logits.stride(0), ids.data_ptr(), ids.stride(0), t,
+                                     unfinished.data_ptr(), pad_id, eos_id, float(temperature), int(top_k), float(top_p),
+                                     seed.data_ptr()))
+
+
 def t5_attention_bwd(q, k, v, ctx, dctx, lse, dq, dk_, dv, B, H, Lq, Lk, dk, *, bias_table=None, lut=None, rel_zero=0,
                      num_buckets=32, causal=False, q_offset=0, dbias_table=None, dropout_p=0.0, seed=0, seed_ptr=None):
     """dq / dk_ / dv are preallocated outputs with the same row strides as q / k / v."""
