@@ -282,6 +282,17 @@ int klab_dropout_apply(void* stream, int dtype, long long n, const void* x, void
  * with fresh masks and without a host round trip. */
 int klab_seed_advance(void* stream, unsigned long long* seed_counter);
 
+/* Gated-GELU feed-forward of T5 v1.1 / Flan-T5 (T5DenseGatedActDense, HF/models/t5/modeling_t5.py:106-132), elementwise part.
+ * u [rows, 2*d_ff] contiguous = [a | b], the output of ONE GEMM against the [wi_0; wi_1] operand.
+ * fwd: h [rows, d_ff] = dropout(gelu_new(a) * b), gelu_new(x) = 0.5 x (1 + tanh(sqrt(2/pi) (x + 0.044715 x^3))).
+ * bwd: du [rows, 2*d_ff] = [dh' * b * gelu_new'(a) | dh' * gelu_new(a)] with dh' = dropout(dh).
+ * The mask is the one klab_dropout_apply(p, seed, seed_ptr) draws for a contiguous [rows, d_ff] tensor.  bf16 or fp32 in and
+ * out, fp32 arithmetic; d_ff must be a multiple of 8 and every pointer 16-byte aligned (KLAB_ERR_INVALID otherwise). */
+int klab_geglu_fwd(void* stream, int dtype, long long rows, int d_ff, const void* u, void* h, float p, unsigned long long seed,
+                   const unsigned long long* seed_ptr);
+int klab_geglu_bwd(void* stream, int dtype, long long rows, int d_ff, const void* dh, const void* u, void* du, float p,
+                   unsigned long long seed, const unsigned long long* seed_ptr);
+
 /* ---- N1: fused multi-tensor Adam (the optimizer step that follows the path: /root/reference/train.py:28,66,
  * torch.optim.Adam over model.transformer.parameters(); semantics of torch/optim/adam.py with amsgrad = False).
  * table (DEVICE, int64 [n_tensors][6]) = {param fp32*, grad fp32*, exp_avg fp32*, exp_avg_sq fp32*, bf16 operand copy* or 0,

@@ -95,6 +95,8 @@ SIGNATURES = {
     "klab_beam_update": [_vp, _i, _i, _i, _i, _i, _i, _f, _i, _vp, _vp, _vp, _vp, _vp, _ll, _vp, _vp, _vp, _vp, _vp, _vp, _vp],
     "klab_dropout_apply": [_vp, _i, _ll, _vp, _vp, _f, _ull, _vp],
     "klab_seed_advance": [_vp, _vp],
+    "klab_geglu_fwd": [_vp, _i, _ll, _i, _vp, _vp, _f, _ull, _vp],
+    "klab_geglu_bwd": [_vp, _i, _ll, _i, _vp, _vp, _vp, _f, _ull, _vp],
     "klab_adam_chunk_elems": [],
     "klab_adam_step": [_vp, _vp, _vp, _i, _d, _d, _d, _d, _d, _ll, _d],
 }

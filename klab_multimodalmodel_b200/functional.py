@@ -364,17 +364,26 @@ def _t5_attn_bwd(c, dh, n, kv_src, wq_or_qkv, wkv, wo, qkv, kvbuf, ctxt, lse, ta
 
 
 def _t5_ff_fwd(c, x, ln_w, wi, wo, seed):
+    """-> (out, n, rstd, f) or, gated, (out, n, rstd, f, u).  wi: the [wi] or [wi_0; wi_1] operand."""
     n, rstd = O.rmsnorm_fwd(x, ln_w, c.eps)
-    f = O.linear_fwd(n, wi, act=L.ACT_RELU, dropout_p=c.p, seed=seed, seed_ptr=c.seed_ptr)
+    if c.gated:                                          # T5DenseGatedActDense (:106-132): one GEMM for both projections
+        u = O.linear_fwd(n, wi)
+        f = O.geglu_fwd(u, c.p, seed, c.seed_ptr)
+    else:
+        f = O.linear_fwd(n, wi, act=L.ACT_RELU, dropout_p=c.p, seed=seed, seed_ptr=c.seed_ptr)
     out = O.linear_fwd(f, wo, residual=x, dropout_p=c.p, seed=seed + 1, seed_ptr=c.seed_ptr)
-    return out, n, rstd, f
+    return (out, n, rstd, f, u) if c.gated else (out, n, rstd, f)
 
 
-def _t5_ff_bwd(c, dout, x, ln_w, wi, wo, n, rstd, f, seed, next_seed, g_ln=None, g_wi=None, g_wo=None):
+def _t5_ff_bwd(c, dout, x, ln_w, wi, wo, n, rstd, f, seed, next_seed, g_ln=None, g_wi=None, g_wo=None, u=None):
     """next_seed: dropout seed of the sub-layer that consumes dx (its output-dropout mask is applied in the same pass).
-    -> dx, dropout(dx) or None, dln, dwi, dwo"""
+    u: the saved [a | b] of the gated FFN.  -> dx, dropout(dx) or None, dln, dwi, dwo"""
     dy = O.dropout_apply(dout, c.p, seed + 1, c.seed_ptr) if c.p > 0.0 else dout
-    df = O.linear_dgrad(dy, wo, act=L.ACT_RELU_BWD, aux_in=f, dropout_p=c.p, seed=seed, seed_ptr=c.seed_ptr)
+    if c.gated:
+        dh = O.linear_dgrad(dy, wo)
+        df = O.geglu_bwd(dh, u, c.p, seed, c.seed_ptr)   # [d a | d b]: one dgrad and one wgrad GEMM against [wi_0; wi_1]
+    else:
+        df = O.linear_dgrad(dy, wo, act=L.ACT_RELU_BWD, aux_in=f, dropout_p=c.p, seed=seed, seed_ptr=c.seed_ptr)
     dwo = _wgrad(dy, f, out=g_wo)
     dn = O.linear_dgrad(df, wi)
     dwi = _wgrad(df, n, out=g_wi)
@@ -386,17 +395,17 @@ def _t5_ff_bwd(c, dout, x, ln_w, wi, wo, n, rstd, f, seed, next_seed, g_ln=None,
 
 
 def _t5_operands(c, params, cd, mode):
-    """(wqkv, w_o, w_i, w_ff[, w_cq, w_ckv, w_co]) in the compute dtype; mode in {"get", "peek"}."""
+    """(wqkv, w_o, w_i, w_ff[, w_cq, w_ckv, w_co]) in the compute dtype; mode in {"get", "peek"}.  Gated: w_i = [wi_0; wi_1]."""
     f = getattr(c.cache, mode)
     if c.is_decoder:
-        ln0, q, k, v, o, ln1, cq, ck, cv, co, ln2, wi, wo = params
-        return f([q, k, v], cd), f([o], cd), f([wi], cd), f([wo], cd), f([cq], cd), f([ck, cv], cd), f([co], cd)
-    ln0, q, k, v, o, ln1, wi, wo = params
-    return f([q, k, v], cd), f([o], cd), f([wi], cd), f([wo], cd)
+        ln0, q, k, v, o, ln1, cq, ck, cv, co, ln2, *wi, wo = params
+        return f([q, k, v], cd), f([o], cd), f(wi, cd), f([wo], cd), f([cq], cd), f([ck, cv], cd), f([co], cd)
+    ln0, q, k, v, o, ln1, *wi, wo = params
+    return f([q, k, v], cd), f([o], cd), f(wi, cd), f([wo], cd)
 
 
 def _t5_block_fwd_body(x, enc_out, c, save, table, *params):
-    """-> (out,) or (out, n0, rstd0, qkv, ctx, lse, h1, [n1, rstd1, qc, kvbuf, ctx2, lse2, h2,] n2, rstd2, f)"""
+    """-> (out,) or (out, n0, rstd0, qkv, ctx, lse, h1, [n1, rstd1, qc, kvbuf, ctx2, lse2, h2,] n2, rstd2, f[, u]); u: gated FFN"""
     cd = x.dtype
     dec = c.is_decoder
     ws = _t5_operands(c, params, cd, "peek")
@@ -415,17 +424,20 @@ def _t5_block_fwd_body(x, enc_out, c, save, table, *params):
         n1, rstd1 = O.rmsnorm_fwd(h1, ln1, c.eps)
         h2, qc, kvbuf, ctx2, lse2 = _t5_attn_fwd(c, n1, enc_out, w_cq, w_ckv, w_co, h1, None, None, 0, False, c.L, c.Le, seed + 2,
                                                  kvbuf=kv_pre)
-        out, n2, rstd2, f = _t5_ff_fwd(c, h2, ln2, w_i, w_ff, seed + 4)
-        return (out, n0, rstd0, qkv, ctxt, lse, h1, n1, rstd1, qc, kvbuf, ctx2, lse2, h2, n2, rstd2, f) if save else (out,)
-    out, n2, rstd2, f = _t5_ff_fwd(c, h1, ln1, w_i, w_ff, seed + 4)
-    return (out, n0, rstd0, qkv, ctxt, lse, h1, n2, rstd2, f) if save else (out,)
+        out, *ff = _t5_ff_fwd(c, h2, ln2, w_i, w_ff, seed + 4)
+        return (out, n0, rstd0, qkv, ctxt, lse, h1, n1, rstd1, qc, kvbuf, ctx2, lse2, h2, *ff) if save else (out,)
+    out, *ff = _t5_ff_fwd(c, h1, ln1, w_i, w_ff, seed + 4)
+    return (out, n0, rstd0, qkv, ctxt, lse, h1, *ff) if save else (out,)
 
 
 def _t5_block_bwd_body(dout, x, enc_out, *rest):
     """rest = saved activations (forward order) then consts (c, table, *params)
     -> (dx, denc | None, dtable | None, *param grads, flat): every parameter gradient is a slice of `flat` (see _flat_grads)"""
     n_acts = 16 if enc_out is not None else 9
+    if not isinstance(rest[n_acts], Ctx):                # the gated FFN saves u as well
+        n_acts += 1
     acts, (c, table, *params) = rest[:n_acts], rest[n_acts:]
+    u = acts[n_acts - 1] if c.gated else None
     cd = x.dtype
     dec = c.is_decoder
     ws = _t5_operands(c, params, cd, "peek")
@@ -435,12 +447,13 @@ def _t5_block_bwd_body(dout, x, enc_out, *rest):
     dtable = torch.zeros_like(table) if table is not None else None
     denc = None
     if dec:
-        n0, rstd0, qkv, ctxt, lse, h1, n1, rstd1, qc, kvbuf, ctx2, lse2, h2, n2, rstd2, f = acts
+        n0, rstd0, qkv, ctxt, lse, h1, n1, rstd1, qc, kvbuf, ctx2, lse2, h2, n2, rstd2, f = acts[:16]
         ln0, ln1, ln2 = params[0], params[5], params[10]
         wqkv, w_o, w_i, w_ff, w_cq, w_ckv, w_co = ws
         flat, (g_ln0, g_qkv, g_o, g_ln1, g_cq, g_ckv, g_co, g_ln2, g_wi, g_ff) = _flat_grads(
             [(d,), (3 * inner, d), (d, inner), (d,), (inner, d), (2 * inner, d), (d, inner), (d,), tuple(w_i.shape), tuple(w_ff.shape)], x.device)
-        dh2, dh2d, dln2, dwi, dwo_ff = _t5_ff_bwd(c, dout, h2, ln2, w_i, w_ff, n2, rstd2, f, seed + 4, seed + 2, g_ln=g_ln2, g_wi=g_wi, g_wo=g_ff)
+        dh2, dh2d, dln2, dwi, dwo_ff = _t5_ff_bwd(c, dout, h2, ln2, w_i, w_ff, n2, rstd2, f, seed + 4, seed + 2, g_ln=g_ln2, g_wi=g_wi, g_wo=g_ff,
+                                                  u=u)
         dn1, denc, dwcq, dwckv, dwco = _t5_attn_bwd(c, dh2, n1, enc_out, w_cq, w_ckv, w_co, qc, kvbuf, ctx2, lse2, None, None, 0,
                                                     False, c.L, c.Le, seed + 2, None, dh_dropped=dh2d, g_wq=g_cq, g_wkv=g_ckv, g_wo=g_co)
         if c.p > 0.0:                                    # + the self-attention layer's output-dropout mask for its backward
@@ -448,28 +461,31 @@ def _t5_block_bwd_body(dout, x, enc_out, *rest):
         else:
             (dh1, dln1), dh1d = O.rmsnorm_bwd(dn1, h1, ln1, rstd1, dres=dh2, dgamma_out=g_ln1), None
     else:
-        n0, rstd0, qkv, ctxt, lse, h1, n2, rstd2, f = acts
+        n0, rstd0, qkv, ctxt, lse, h1, n2, rstd2, f = acts[:9]
         ln0, ln1 = params[0], params[5]
         wqkv, w_o, w_i, w_ff = ws
         flat, (g_ln0, g_qkv, g_o, g_ln1, g_wi, g_ff) = _flat_grads(
             [(d,), (3 * inner, d), (d, inner), (d,), tuple(w_i.shape), tuple(w_ff.shape)], x.device)
-        dh1, dh1d, dln1, dwi, dwo_ff = _t5_ff_bwd(c, dout, h1, ln1, w_i, w_ff, n2, rstd2, f, seed + 4, seed, g_ln=g_ln1, g_wi=g_wi, g_wo=g_ff)
+        dh1, dh1d, dln1, dwi, dwo_ff = _t5_ff_bwd(c, dout, h1, ln1, w_i, w_ff, n2, rstd2, f, seed + 4, seed, g_ln=g_ln1, g_wi=g_wi, g_wo=g_ff,
+                                                  u=u)
     dn0, _, dwqkv, _, dwo = _t5_attn_bwd(c, dh1, n0, None, wqkv, None, w_o, qkv, None, ctxt, lse, table, c.lut, c.rz, dec,
                                          c.L, c.L, seed, dtable, dh_dropped=dh1d, g_wq=g_qkv, g_wo=g_o)
     dx, dln0 = O.rmsnorm_bwd(dn0, x, ln0, rstd0, dres=dh1, dgamma_out=g_ln0)
     _Side.join()
     gq, gk, gv = dwqkv[:inner], dwqkv[inner:2 * inner], dwqkv[2 * inner:]
+    gwi = (dwi[:dwi.shape[0] // 2], dwi[dwi.shape[0] // 2:]) if c.gated else (dwi,)      # gated: wi_0 | wi_1
     if dec:
-        grads = (dln0, gq, gk, gv, dwo, dln1, dwcq, dwckv[:inner], dwckv[inner:], dwco, dln2, dwi, dwo_ff)
+        grads = (dln0, gq, gk, gv, dwo, dln1, dwcq, dwckv[:inner], dwckv[inner:], dwco, dln2, *gwi, dwo_ff)
     else:
-        grads = (dln0, gq, gk, gv, dwo, dln1, dwi, dwo_ff)
+        grads = (dln0, gq, gk, gv, dwo, dln1, *gwi, dwo_ff)
     return (dx, denc, dtable) + grads + (flat,)
 
 
 class T5BlockFn(torch.autograd.Function):
     """One T5Block.  inputs: (c, x, enc_out | None, bias_table | None, *params)
     params (encoder): ln0, q, k, v, o, ln1, wi, wo
-    params (decoder): ln0, q, k, v, o, ln1, cq, ck, cv, co, ln2, wi, wo"""
+    params (decoder): ln0, q, k, v, o, ln1, cq, ck, cv, co, ln2, wi, wo
+    (gated FFN: wi_0, wi_1 in place of wi)"""
 
     @staticmethod
     def forward(ctx, c, x, enc_out, table, *params):
@@ -599,8 +615,9 @@ LMHEAD_VOCAB_CHUNK = 8192      # backward recomputes the logits this many vocabu
 
 
 class LMHeadLossFn(torch.autograd.Function):
-    """final RMSNorm -> dropout (training) -> * d_model**-0.5 -> tied LM head -> CrossEntropyLoss(ignore_index=-100),
-    HF/models/t5/modeling_t5.py:767-768,1105-1117.
+    """final RMSNorm -> dropout (training) -> * alpha -> LM head -> CrossEntropyLoss(ignore_index=-100),
+    HF/models/t5/modeling_t5.py:767-768,1105-1117.  alpha = d_model**-0.5, or 1 for T5 v1.1 (config.scale_decoder_outputs);
+    `table` is lm_head.weight (shared.weight itself when tied).
 
     bf16 (hot path): the LM-head GEMM is fused with the cross entropy and vocab-tiled -- its epilogue reduces every 128 x 256
     logits tile to online-softmax partials straight out of TMEM, so the [rows, 32128] logits are never written; backward
@@ -609,7 +626,7 @@ class LMHeadLossFn(torch.autograd.Function):
     fp32 (strict parity path): materialised logits + klab_ce_fwd / klab_ce_bwd."""
 
     @staticmethod
-    def forward(ctx, x, ln_w, table, labels, cache, eps, p, seed, seed_ptr):
+    def forward(ctx, x, ln_w, table, labels, cache, eps, p, seed, seed_ptr, alpha):
         cd = x.dtype
         V, d = table.shape
         tab = cache.get([table], cd)
@@ -620,14 +637,14 @@ class LMHeadLossFn(torch.autograd.Function):
         fused = cd == torch.bfloat16
         if fused:
             logits, vpad = None, 0
-            lse, stats = O.lmhead_ce_fwd(n, tab, d ** -0.5, lab)
+            lse, stats = O.lmhead_ce_fwd(n, tab, alpha, lab)
         else:
             vpad = (V + 7) // 8 * 8
-            logits = O.linear_fwd(n, tab, alpha=d ** -0.5, ldd_pad=vpad)
+            logits = O.linear_fwd(n, tab, alpha=alpha, ldd_pad=vpad)
             lse, stats = O.ce_fwd(logits, V, lab)
         if _needs_grad((x, ln_w, table)):
             ctx.save_for_backward(x, ln_w, table, lab, rstd, n, logits, lse, stats)
-            ctx.cache, ctx.vpad, ctx.p, ctx.seed, ctx.seed_ptr, ctx.fused = cache, vpad, p, seed, seed_ptr, fused
+            ctx.cache, ctx.vpad, ctx.p, ctx.seed, ctx.seed_ptr, ctx.fused, ctx.alpha = cache, vpad, p, seed, seed_ptr, fused, alpha
             ctx.step_token = _StepToken()
         return stats[0].clone()
 
@@ -639,7 +656,7 @@ class LMHeadLossFn(torch.autograd.Function):
         V, d = table.shape
         tab = ctx.cache.get([table], x.dtype)
         g = gloss.reshape(1).to(torch.float32).contiguous()
-        alpha = d ** -0.5
+        alpha = ctx.alpha
         if ctx.fused:
             rows = n.shape[0]
             chunk = min(LMHEAD_VOCAB_CHUNK, (V + 7) // 8 * 8)
@@ -659,7 +676,7 @@ class LMHeadLossFn(torch.autograd.Function):
         if ctx.p > 0.0:
             dn = O.dropout_apply(dn, ctx.p, ctx.seed, ctx.seed_ptr)
         dx, dln = O.rmsnorm_bwd(dn, x, ln_w, rstd)
-        return dx, dln, dtab, None, None, None, None, None, None
+        return dx, dln, dtab, None, None, None, None, None, None, None
 
 
 # ------------------------------------------------------------------------------------------------

@@ -42,14 +42,30 @@ class _DecodeState:
         self.lut, self.rz = tr.decoder.lut(T, dev)                 # covers relative positions -(T-1) .. T-1
 
 
-def _decode_operands(tr, cd):
-    g = tr.cache.get                                               # refreshes stale bf16 copies eagerly (outside any graph)
+def _decode_operands(tr, cd, mode="get"):
+    """-> (per decoder block (ln0, wqkv, w_o, ln1, w_cq, w_ckv, w_co, ln2, w_i, w_ff), embedding table, LM head) in the compute
+    dtype.  "get" refreshes stale bf16 copies eagerly (outside any graph); "peek" returns the buffers as they are.  The LM head
+    is the embedding operand itself when tied; w_i is [wi_0; wi_1] for the gated FFN."""
+    g = getattr(tr.cache, mode)
     out = []
     for blk in tr.decoder.block:
-        ln0, q, k, v, o, ln1, cq, ck, cv, co, ln2, wi, wo = blk.flat_params()
+        ln0, q, k, v, o, ln1, cq, ck, cv, co, ln2, *wi, wo = blk.flat_params()
         out.append((ln0.detach(), g([q, k, v], cd), g([o], cd), ln1.detach(), g([cq], cd), g([ck, cv], cd), g([co], cd), ln2.detach(),
-                    g([wi], cd), g([wo], cd)))
-    return out, g([tr.shared.weight], cd)
+                    g(wi, cd), g([wo], cd)))
+    return out, g([tr.shared.weight], cd), g([tr.lm_head.weight], cd)
+
+
+def _decode_operands_peek(tr, cd):
+    return _decode_operands(tr, cd, "peek")
+
+
+def _ffn(cfg, n2, w_i, w_ff, h2):
+    """Decoder FFN of one token per row, eval mode: ReLU (T5DenseActDense) or gated-GELU (T5DenseGatedActDense)."""
+    if cfg.gated:
+        f = O.geglu_fwd(O.linear_fwd(n2, w_i))
+    else:
+        f = O.linear_fwd(n2, w_i, act=L.ACT_RELU)
+    return O.linear_fwd(f, w_ff, residual=h2)
 
 
 def _decode_step_body(tr, st, t, B, Le, T, sample=None):
@@ -61,9 +77,9 @@ def _decode_step_body(tr, st, t, B, Le, T, sample=None):
     n_rs = 1 if sample is None else sample[0]
     R = B * n_rs
     cd = st.enc.dtype
-    H, dk, d, eps = cfg.num_heads, cfg.d_kv, cfg.d_model, cfg.layer_norm_epsilon
+    H, dk, eps = cfg.num_heads, cfg.d_kv, cfg.layer_norm_epsilon
     inner = H * dk
-    layers, tab = _decode_operands_peek(tr, cd)
+    layers, tab, head = _decode_operands_peek(tr, cd)
     table = tr.decoder.block[0].layer[0].SelfAttention.relative_attention_bias.weight.detach()
     st.tok.copy_(st.ids[:, t:t + 1])
     x = O.embedding_fwd(st.tok, tab)                               # [R, d]
@@ -84,10 +100,9 @@ def _decode_step_body(tr, st, t, B, Le, T, sample=None):
             ctx2 = O.t5_attention_decode_beam(qc, cross_kv[:, :inner], cross_kv[:, inner:], R, H, Le, dk, kv_group=n_rs)
         h2 = O.linear_fwd(ctx2, w_co, residual=h1)
         n2, _ = O.rmsnorm_fwd(h2, ln2, eps, save_stats=False)
-        f = O.linear_fwd(n2, w_i, act=L.ACT_RELU)
-        x = O.linear_fwd(f, w_ff, residual=h2)
+        x = _ffn(cfg, n2, w_i, w_ff, h2)
     n, _ = O.rmsnorm_fwd(x, tr.decoder.final_layer_norm.weight, eps, save_stats=False)
-    logits = O.linear_fwd(n, tab, alpha=d ** -0.5, out_dtype=torch.float32)
+    logits = O.linear_fwd(n, head, alpha=cfg.lm_head_scale, out_dtype=torch.float32)
     if sample is None:
         L.check(L.lib().klab_greedy_step(torch.cuda.current_stream().cuda_stream, B, tr.shared.weight.shape[0], logits.data_ptr(),
                                          logits.stride(0), st.ids.data_ptr(), st.ids.stride(0), t + 1, st.unfinished.data_ptr(),
@@ -97,16 +112,6 @@ def _decode_step_body(tr, st, t, B, Le, T, sample=None):
         O.sample_step(logits, st.ids, t + 1, st.unfinished, st.seed, pad_id=cfg.pad_token_id, eos_id=cfg.eos_token_id,
                       temperature=temperature, top_k=top_k, top_p=top_p)
     return (st.ids,)
-
-
-def _decode_operands_peek(tr, cd):
-    pk = tr.cache.peek
-    out = []
-    for blk in tr.decoder.block:
-        ln0, q, k, v, o, ln1, cq, ck, cv, co, ln2, wi, wo = blk.flat_params()
-        out.append((ln0.detach(), pk([q, k, v], cd), pk([o], cd), ln1.detach(), pk([cq], cd), pk([ck, cv], cd), pk([co], cd), ln2.detach(),
-                    pk([wi], cd), pk([wo], cd)))
-    return out, pk([tr.shared.weight], cd)
 
 
 CHECK_EVERY = 5           # decode steps between two read-backs of the "every row has finished" flag
@@ -133,7 +138,7 @@ def _decode_run(tr, st, embeds, B, Le, T, key, sample=None):
     cd = embeds.dtype
     enc = tr.encoder.run_blocks(embeds, B, Le, tr.cache)
     O.rmsnorm_fwd(enc, tr.encoder.final_layer_norm.weight, cfg.layer_norm_epsilon, out=st.enc, save_stats=False)
-    layers, _ = _decode_operands(tr, cd)                                 # also validates / refreshes every operand copy
+    layers, _, _ = _decode_operands(tr, cd)                                 # also validates / refreshes every operand copy
     for l, ops_l in enumerate(layers):
         O.linear_fwd(st.enc, ops_l[5], out=st.cross_kv[l])               # cross k|v, once per caption batch (modeling_t5.py:291-299)
     st.ids.fill_(cfg.pad_token_id)
@@ -174,7 +179,7 @@ def greedy_generate_recompute(tr, embeds, B, Le, max_new_tokens: int = 20):
     dev = embeds.device
     enc = tr.encoder.run_blocks(embeds, B, Le, tr.cache)
     enc, _ = O.rmsnorm_fwd(enc, tr.encoder.final_layer_norm.weight, cfg.layer_norm_epsilon, save_stats=False)
-    tab = tr.cache.get([tr.shared.weight], cd)
+    tab, head = tr.cache.get([tr.shared.weight], cd), tr.cache.get([tr.lm_head.weight], cd)
     V, d = tr.shared.weight.shape
     ids = torch.full((B, max_new_tokens + 1), cfg.pad_token_id, dtype=torch.int64, device=dev)
     ids[:, 0] = cfg.decoder_start_token_id
@@ -187,7 +192,7 @@ def greedy_generate_recompute(tr, embeds, B, Le, max_new_tokens: int = 20):
         x = tr.decoder.run_blocks(x, B, Lt, tr.cache, enc_out=enc, Le=Le)
         last = x.view(B, Lt, d)[:, -1, :]                               # strided rows: the norm kernel takes a row stride
         n, _ = O.rmsnorm_fwd(last, tr.decoder.final_layer_norm.weight, cfg.layer_norm_epsilon, save_stats=False)
-        logits = O.linear_fwd(n, tab, alpha=d ** -0.5, out_dtype=torch.float32)
+        logits = O.linear_fwd(n, head, alpha=cfg.lm_head_scale, out_dtype=torch.float32)
         L.check(L.lib().klab_greedy_step(torch.cuda.current_stream().cuda_stream, B, V, logits.data_ptr(), logits.stride(0),
                                          ids.data_ptr(), ids.stride(0), Lt, unfinished.data_ptr(), cfg.pad_token_id, cfg.eos_token_id))
         n_out = Lt + 1
@@ -252,11 +257,11 @@ def _beam_step_body(tr, st, t, B, nb, Le, T, length_penalty, early_stopping):
     """Position t for every hypothesis, then top-k and the beam update.  Reads and writes `st` and the operand cache only."""
     cfg = tr.config
     cd = st.enc.dtype
-    H, dk, d, eps = cfg.num_heads, cfg.d_kv, cfg.d_model, cfg.layer_norm_epsilon
+    H, dk, eps = cfg.num_heads, cfg.d_kv, cfg.layer_norm_epsilon
     inner = H * dk
     R = B * nb
     V = tr.shared.weight.shape[0]
-    layers, tab = _decode_operands_peek(tr, cd)
+    layers, tab, head = _decode_operands_peek(tr, cd)
     table = tr.decoder.block[0].layer[0].SelfAttention.relative_attention_bias.weight.detach()
     src = st.src[t & 1]
     x = O.embedding_fwd(st.next_tok, tab)                          # [R, d]
@@ -273,10 +278,9 @@ def _beam_step_body(tr, st, t, B, nb, Le, T, length_penalty, early_stopping):
         ctx2 = O.t5_attention_decode_beam(qc, cross_kv[:, :inner], cross_kv[:, inner:], R, H, Le, dk, kv_group=nb)
         h2 = O.linear_fwd(ctx2, w_co, residual=h1)
         n2, _ = O.rmsnorm_fwd(h2, ln2, eps, save_stats=False)
-        f = O.linear_fwd(n2, w_i, act=L.ACT_RELU)
-        x = O.linear_fwd(f, w_ff, residual=h2)
+        x = _ffn(cfg, n2, w_i, w_ff, h2)
     n, _ = O.rmsnorm_fwd(x, tr.decoder.final_layer_norm.weight, eps, save_stats=False)
-    logits = O.linear_fwd(n, tab, alpha=d ** -0.5, out_dtype=torch.float32)
+    logits = O.linear_fwd(n, head, alpha=cfg.lm_head_scale, out_dtype=torch.float32)
     lib, stream = L.lib(), torch.cuda.current_stream().cuda_stream
     K = 2 * nb
     L.check(lib.klab_beam_topk(stream, R, V, K, logits.data_ptr(), logits.stride(0), st.run_scores.data_ptr(), st.cand_val.data_ptr(),
@@ -309,7 +313,7 @@ def beam_generate(tr, embeds, B, Le, num_beams: int, max_new_tokens: int = 20, l
         st = states[key] = _BeamState(tr, B, nb, Le, T, cd, dev)
     enc = tr.encoder.run_blocks(embeds, B, Le, tr.cache)
     O.rmsnorm_fwd(enc, tr.encoder.final_layer_norm.weight, cfg.layer_norm_epsilon, out=st.enc, save_stats=False)
-    layers, _ = _decode_operands(tr, cd)
+    layers, _, _ = _decode_operands(tr, cd)
     for l, ops_l in enumerate(layers):
         O.linear_fwd(st.enc, ops_l[5], out=st.cross_kv[l])
     st.reset(cfg, nb)

@@ -43,6 +43,11 @@ class T5Config:
     pad_token_id: int = 0
     eos_token_id: int = 1
     decoder_start_token_id: int = 0
+    tie_word_embeddings: bool = True
+    # HF/models/t5/configuration_t5.py:79-83: T5 v1.1 checkpoints say `"tie_word_embeddings": false`, and that is what switches the
+    # d_model ** -0.5 scale in front of the LM head off (modeling_t5.py:1107).  None: derived from tie_word_embeddings as HF does;
+    # a config.json that transformers wrote stores the derived value itself.
+    scale_decoder_outputs: bool | None = None
 
     NAMED = {
         "t5-small": dict(d_model=512, d_ff=2048, num_layers=6, num_heads=8),
@@ -50,7 +55,30 @@ class T5Config:
         "t5-large": dict(d_model=1024, d_ff=4096, num_layers=24, num_heads=16),
         "t5-3b": dict(d_model=1024, d_kv=128, d_ff=16384, num_layers=24, num_heads=32),
         "t5-11b": dict(d_model=1024, d_kv=128, d_ff=65536, num_layers=24, num_heads=128),
+        **{f"google/{family}-{size}": dict(arch, feed_forward_proj="gated-gelu", tie_word_embeddings=False)
+           for family in ("flan-t5", "t5-v1_1")
+           for size, arch in (("small", dict(d_model=512, d_ff=1024, num_layers=8, num_heads=6)),
+                              ("base", dict(d_model=768, d_ff=2048, num_layers=12, num_heads=12)),
+                              ("large", dict(d_model=1024, d_ff=2816, num_layers=24, num_heads=16)))},
     }
+    FEED_FORWARD_PROJ = ("relu", "gated-gelu")
+
+    def __post_init__(self):
+        if self.feed_forward_proj not in self.FEED_FORWARD_PROJ:
+            raise ValueError(f"T5Config: feed_forward_proj={self.feed_forward_proj!r} is not supported (supported: "
+                             f"{', '.join(self.FEED_FORWARD_PROJ)})")
+        if self.scale_decoder_outputs is None:
+            self.scale_decoder_outputs = self.tie_word_embeddings is not False
+
+    @property
+    def gated(self) -> bool:
+        """T5 v1.1 / Flan-T5 feed-forward: h = gelu_new(x wi_0^T) * (x wi_1^T) (HF/models/t5/modeling_t5.py:106-132)."""
+        return self.feed_forward_proj == "gated-gelu"
+
+    @property
+    def lm_head_scale(self) -> float:
+        """Factor on the final decoder state in front of the LM head (HF/models/t5/modeling_t5.py:1107)."""
+        return self.d_model ** -0.5 if self.scale_decoder_outputs else 1.0
 
     @property
     def n_dec(self):
@@ -155,11 +183,13 @@ def _config_from_source(cls, source, **overrides):
 _BASE_PREFIXES = ("swinv2.", "transformer.", "model.", "encoder_model.")
 
 
-def _load_checkpoint_dir(module: nn.Module, path: str) -> None:
+def _load_checkpoint_dir(module: nn.Module, path: str, before_load=None) -> None:
     """Load model.safetensors / pytorch_model.bin of a checkpoint directory, strict on the module's own keys.  Like HF's
     `from_pretrained` it strips the base-model prefix when the file was written by a task head (the published
     microsoft/swinv2-* checkpoints are Swinv2ForImageClassification: 'swinv2.embeddings...' + 'classifier.*') and reports the
-    keys it drops.  A directory without weights is an error: the reference never random-initialises silently."""
+    keys it drops.  A directory without weights is an error: the reference never random-initialises silently.
+    before_load(sd): called with the file's tensors before tied keys are filled in (T5ForConditionalGeneration unties its LM
+    head there when the file holds a distinct one)."""
     st = os.path.join(path, "model.safetensors")
     pt = os.path.join(path, "pytorch_model.bin")
     if os.path.exists(st):
@@ -176,6 +206,9 @@ def _load_checkpoint_dir(module: nn.Module, path: str) -> None:
             if any(k in own for k in stripped):
                 sd = {**{k: v for k, v in sd.items() if not k.startswith(pre)}, **stripped}
                 break
+    if before_load is not None:
+        before_load(sd)
+        own = module.state_dict()
     for k in own:                      # tied tensors are stored once in safetensors files
         if k not in sd:
             for alias in ("shared.weight", "encoder.embed_tokens.weight", "decoder.embed_tokens.weight", "lm_head.weight"):
@@ -243,9 +276,19 @@ class _T5CrossLayer(nn.Module):
 
 
 class _T5Dense(nn.Module):
+    """T5DenseActDense (wi, wo) or, gated, T5DenseGatedActDense (wi_0, wi_1, wo); HF keeps the name DenseReluDense for both."""
+
     def __init__(self, cfg):
         super().__init__()
-        self.wi, self.wo = _P(cfg.d_ff, cfg.d_model), _P(cfg.d_model, cfg.d_ff)
+        if cfg.gated:
+            self.wi_0, self.wi_1 = _P(cfg.d_ff, cfg.d_model), _P(cfg.d_ff, cfg.d_model)
+        else:
+            self.wi = _P(cfg.d_ff, cfg.d_model)
+        self.wo = _P(cfg.d_model, cfg.d_ff)
+
+    def in_weights(self):
+        """[wi] or [wi_0, wi_1]: the blocks of the one input-projection operand."""
+        return [self.wi_0.weight, self.wi_1.weight] if hasattr(self, "wi_0") else [self.wi.weight]
 
 
 class _T5FFLayer(nn.Module):
@@ -274,7 +317,7 @@ class _T5Block(nn.Module):
             ps += [ca.layer_norm.weight, ca.EncDecAttention.q.weight, ca.EncDecAttention.k.weight, ca.EncDecAttention.v.weight,
                    ca.EncDecAttention.o.weight]
         ff = self.layer[-1]
-        ps += [ff.layer_norm.weight, ff.DenseReluDense.wi.weight, ff.DenseReluDense.wo.weight]
+        ps += [ff.layer_norm.weight, *ff.DenseReluDense.in_weights(), ff.DenseReluDense.wo.weight]
         return ps
 
 
@@ -309,7 +352,7 @@ class T5Stack(nn.Module):
         if c is None:
             cfg = self.cfg
             lut, rz = self.lut(L_, device)
-            c = self._ctxs[key] = Ctx(cache=cache, is_decoder=self.is_decoder, B=B, L=L_, Le=Le, H=cfg.num_heads, dk=cfg.d_kv,
+            c = self._ctxs[key] = Ctx(cache=cache, is_decoder=self.is_decoder, gated=cfg.gated, B=B, L=L_, Le=Le, H=cfg.num_heads, dk=cfg.d_kv,
                                       eps=cfg.layer_norm_epsilon, num_buckets=cfg.relative_attention_num_buckets, lut=lut, rz=rz, p=p,
                                       seed=self.seed_base + 16 * (i + 1), seed_ptr=step_seed(device) if p > 0 else None)
         return c
@@ -426,11 +469,32 @@ class T5ForConditionalGeneration(nn.Module):
 
     @classmethod
     def from_pretrained(cls, source, **overrides):
+        """As HF's: a checkpoint whose lm_head.weight differs from shared.weight (T5 v1.1 / Flan-T5 ship their own LM head)
+        gives an untied model whose lm_head holds the file's tensor; equal tensors, or no lm_head.weight, keep them tied."""
         cfg, path = _config_from_source(T5Config, source, **overrides)
         m = cls(cfg)
         if path:
-            _load_checkpoint_dir(m, path)
+            _load_checkpoint_dir(m, path, before_load=m._untie_for)
         return m.eval()
+
+    @property
+    def lm_head_tied(self) -> bool:
+        return self.lm_head.weight is self.shared.weight
+
+    def untie_lm_head(self) -> None:
+        """Give lm_head a parameter of its own (initialised with a copy of shared.weight).  state_dict() keys do not change."""
+        if self.lm_head_tied:
+            self.lm_head.weight = nn.Parameter(self.shared.weight.detach().clone())
+            # captured decode steps baked the tied operand in: drop them with their states
+            from .graphs import POOL
+            POOL.drop_keys(lambda k: len(k) > 1 and k[1] == id(self))
+            for attr in ("_klab_decode_states", "_klab_sample_states", "_klab_beam_states"):
+                self.__dict__.pop(attr, None)
+
+    def _untie_for(self, sd) -> None:
+        head, emb = sd.get("lm_head.weight"), sd.get("shared.weight")
+        if head is not None and emb is not None and head.shape == emb.shape and not torch.equal(head, emb):
+            self.untie_lm_head()
 
     def state_dict(self, *args, **kwargs):
         from .optim import wait_pending_updates
@@ -438,11 +502,14 @@ class T5ForConditionalGeneration(nn.Module):
             wait_pending_updates(self.shared.weight.device if self.shared.weight.is_cuda else None)
         return super().state_dict(*args, **kwargs)
 
-    def load_state_dict(self, *args, **kwargs):
+    def load_state_dict(self, state_dict, *args, **kwargs):
+        """A state dict with a distinct lm_head.weight unties a tied model first (as from_pretrained does), so that
+        MyModel.load of an untied model's file restores both tensors instead of one overwriting the other."""
         from .optim import wait_pending_updates
         if torch.cuda.is_available():
             wait_pending_updates(self.shared.weight.device if self.shared.weight.is_cuda else None)
-        return super().load_state_dict(*args, **kwargs)
+        self._untie_for(state_dict)
+        return super().load_state_dict(state_dict, *args, **kwargs)
 
     def loss_from_embeds(self, embeds, B, Le, labels):
         """embeds: [B*Le, d] encoder inputs_embeds (compute dtype); labels [B, Lt] int64 -> 0-dim fp32 loss
@@ -459,8 +526,8 @@ class T5ForConditionalGeneration(nn.Module):
         labels = labels.contiguous()
         dec_in = Fn.apply_fn(Fn.DecoderEmbedFn, labels, self.shared.weight, self.cache, cd, cfg.decoder_start_token_id, cfg.pad_token_id)
         dec = self.decoder.run_blocks(dec_in, B, Lt, self.cache, enc_out=enc, Le=Le)
-        return Fn.apply_fn(Fn.LMHeadLossFn, dec, self.decoder.final_layer_norm.weight, self.shared.weight, labels, self.cache,
-                           cfg.layer_norm_epsilon, p, self.decoder.seed_base + 7, sp)
+        return Fn.apply_fn(Fn.LMHeadLossFn, dec, self.decoder.final_layer_norm.weight, self.lm_head.weight, labels, self.cache,
+                           cfg.layer_norm_epsilon, p, self.decoder.seed_base + 7, sp, cfg.lm_head_scale)
 
     def generate(self, inputs_embeds=None, return_dict_in_generate=False, output_scores=False, **overrides):
         """`generate(inputs_embeds=[B, Le, d], **overrides)` of HF 5.5.0 for the options in `generation_config`: greedy decoding
@@ -533,7 +600,7 @@ def init_t5_(m: nn.Module, seed: int | None = None):
                 p.normal_(0.0, 1.0, generator=g)
             elif name.endswith(".q.weight"):
                 p.normal_(0.0, (d * dk) ** -0.5, generator=g)
-            elif name.endswith((".k.weight", ".v.weight", "wi.weight", "relative_attention_bias.weight")):
+            elif name.endswith((".k.weight", ".v.weight", "wi.weight", "wi_0.weight", "wi_1.weight", "relative_attention_bias.weight")):
                 p.normal_(0.0, d ** -0.5, generator=g)
             elif name.endswith(".o.weight"):
                 p.normal_(0.0, (h * dk) ** -0.5, generator=g)

@@ -491,6 +491,25 @@ def dropout_apply(x, p, seed, seed_ptr=None):
     return y
 
 
+def geglu_fwd(u, p=0.0, seed=0, seed_ptr=None):
+    """u [rows, 2 d_ff] = [x wi_0^T | x wi_1^T] -> h [rows, d_ff] = dropout(gelu_new(a) * b) (klab_geglu_fwd)."""
+    assert u.is_contiguous() and u.dim() == 2 and u.shape[1] % 2 == 0
+    rows, dff = u.shape[0], u.shape[1] // 2
+    h = torch.empty(rows, dff, dtype=u.dtype, device=u.device)
+    L.check(L.lib().klab_geglu_fwd(_stream(), _DT[u.dtype], rows, dff, u.data_ptr(), h.data_ptr(), float(p), int(seed), _p(seed_ptr)))
+    return h
+
+
+def geglu_bwd(dh, u, p=0.0, seed=0, seed_ptr=None):
+    """-> du [rows, 2 d_ff], the gradient of geglu_fwd (same p / seed / seed_ptr: same mask) w.r.t. u (klab_geglu_bwd)."""
+    dh = dh.contiguous()
+    assert u.is_contiguous() and dh.dtype == u.dtype and tuple(dh.shape) == (u.shape[0], u.shape[1] // 2)
+    du = torch.empty_like(u)
+    L.check(L.lib().klab_geglu_bwd(_stream(), _DT[u.dtype], u.shape[0], u.shape[1] // 2, dh.data_ptr(), u.data_ptr(), du.data_ptr(),
+                                   float(p), int(seed), _p(seed_ptr)))
+    return du
+
+
 def seed_advance(counter: torch.Tensor) -> None:
     """Step the device-side dropout counter (uint64 stored in an int64 tensor) once per training step."""
     L.check(L.lib().klab_seed_advance(_stream(), counter.data_ptr()))
