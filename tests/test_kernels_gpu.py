@@ -203,52 +203,95 @@ def test_norm_grouped_output():
 
 
 # ------------------------------------------------------------------------------------------------ T5 attention
-@pytest.mark.parametrize("dtype", DTYPES)
-@pytest.mark.parametrize("mode,B,H,Lq,Lk,dk", [("enc", 2, 3, 13, 13, 64), ("dec", 2, 2, 9, 9, 64), ("cross", 2, 2, 7, 13, 64),
-                                               ("enc", 1, 2, 81, 81, 16), ("dec", 1, 1, 40, 40, 32),
-                                               ("enc", 2, 2, 96, 96, 64), ("enc", 1, 2, 176, 176, 64), ("dec", 2, 2, 130, 130, 64),
-                                               ("cross", 1, 2, 32, 200, 64), ("cross", 2, 1, 150, 96, 64), ("dec", 3, 2, 32, 32, 64),
-                                               # packed single-tile path: 128 / L problems per tile, partial last tile, both mask kinds
-                                               ("enc", 9, 2, 32, 32, 64), ("dec", 8, 3, 32, 32, 64), ("dec", 5, 3, 64, 64, 64), ("enc", 2, 2, 64, 64, 64),
-                                               # backward kernel choice: 32 x 96 (decoder cross-attention of workload 2a) and 96 x 96 take the two-CTA-per-SM
-                                               # kernel, 128 x 128 / 120 x 100 do not fit twice per SM and take the 512-thread kernel unpacked
-                                               ("cross", 3, 2, 32, 96, 64), ("enc", 2, 2, 128, 128, 64), ("cross", 3, 2, 120, 100, 64), ("dec", 2, 2, 113, 113, 64)])
-def test_t5_attention(dtype, mode, B, H, Lq, Lk, dk):
-    o = ops()
+def _attn_cases(shapes, ps=(0.0, 0.1), multi=False):
+    """pytest params (mode, B, H, Lq, Lk, dk, p, multi); the dropout-free cases keep their plain shape ids."""
+    out = []
+    for shape in shapes:
+        for p in ps:
+            name = "-".join(map(str, shape)) + (f"-p{p}" if p else "") + ("-multi" if multi else "")
+            out.append(pytest.param(*shape, p, multi, id=name))
+    return out
+
+
+# Kernel paths (bf16 needs d_kv = 64 and L <= 256 for tcgen05, everything else runs the generic kernels of t5_attention.cu; fp32
+# always does).  Odd Lk makes the dropout element index (bh*Lq + i)*Lk + j change parity from row to row, which reaches the
+# odd-base branches that rebuild keep bits one element at a time.
+T5_ATTN_SHAPES = [("enc", 2, 3, 13, 13, 64), ("dec", 2, 2, 9, 9, 64), ("cross", 2, 2, 7, 13, 64),
+                  ("enc", 1, 2, 81, 81, 16), ("dec", 1, 1, 40, 40, 32),
+                  ("enc", 2, 2, 96, 96, 64), ("enc", 1, 2, 176, 176, 64), ("dec", 2, 2, 130, 130, 64),
+                  ("cross", 1, 2, 32, 200, 64), ("cross", 2, 1, 150, 96, 64), ("dec", 3, 2, 32, 32, 64),
+                  # packed single-tile path: 128 / L problems per tile, partial last tile, both mask kinds
+                  ("enc", 9, 2, 32, 32, 64), ("dec", 8, 3, 32, 32, 64), ("dec", 5, 3, 64, 64, 64), ("enc", 2, 2, 64, 64, 64),
+                  # backward kernel choice: 32 x 96 (decoder cross-attention of workload 2a) and 96 x 96 take the two-CTA-per-SM
+                  # kernel, 128 x 128 / 120 x 100 do not fit twice per SM and take the 512-thread kernel unpacked
+                  ("cross", 3, 2, 32, 96, 64), ("enc", 2, 2, 128, 128, 64), ("cross", 3, 2, 120, 100, 64), ("dec", 2, 2, 113, 113, 64),
+                  # bf16 generic kernels with L > 256 (odd Lk too); multi-tile tcgen05 kernels with an odd Lk > 128
+                  ("enc", 1, 2, 300, 300, 64), ("cross", 2, 1, 24, 301, 64), ("cross", 2, 2, 40, 139, 64)]
+# the multi-tile tcgen05 kernels forced at single-tile shapes (KLAB_T5_ATTN_MULTI is read on every call)
+T5_ATTN_MULTI_SHAPES = [("enc", 2, 3, 13, 13, 64), ("dec", 5, 3, 64, 64, 64), ("cross", 3, 2, 32, 96, 64), ("dec", 2, 2, 113, 113, 64)]
+
+
+def t5_attention_reference(QKVr, DOr, table, mode, B, H, Lq, Lk, dk, mask=None):
+    """float64 T5 attention (oracle arithmetic, no projections) -> (ctx, lse, dq, dk, dv, dtable | None).  mask: the dropout
+    multipliers [B, H, Lq, Lk] (0 or 65536 / thr16) applied to the probabilities before they meet V."""
     dims = ot5.T5Dims(num_heads=H, d_kv=dk)
     inner = H * dk
-    QKV, QKVr = rnd(B * max(Lq, Lk), 3 * inner, dtype=dtype, seed=1, scale=0.5)
+    QKVd = QKVr.double()
+    qr = QKVd[:B * Lq, :inner].clone().requires_grad_(True)
+    kr = QKVd[:B * Lk, inner:2 * inner].clone().requires_grad_(True)
+    vr = QKVd[:B * Lk, 2 * inner:].clone().requires_grad_(True)
+    tr = table.double().clone().requires_grad_(True)
+    s = qr.view(B, Lq, H, dk).transpose(1, 2) @ kr.view(B, Lk, H, dk).transpose(1, 2).transpose(-1, -2)
+    if mode != "cross":
+        s = s + ot5.t5_bias(tr, Lq, Lk, bidirectional=(mode == "enc"), dims=dims)[None]
+    if mode == "dec":
+        s = s + torch.where(torch.arange(Lk)[None, :] > torch.arange(Lq)[:, None], torch.finfo(torch.float32).min, 0.0).double()
+    p = torch.softmax(s, -1)
+    if mask is not None:
+        p = p * mask
+    ref = (p @ vr.view(B, Lk, H, dk).transpose(1, 2)).transpose(1, 2).reshape(B * Lq, inner)
+    ref.backward(DOr.double())
+    return (ref.detach(), torch.logsumexp(s.detach(), -1), qr.grad, kr.grad, vr.grad,
+            tr.grad if mode != "cross" else None)
+
+
+def t5_attention_case(dtype, mode, B, H, Lq, Lk, dk, p, seed=0, ctr=None, qk_scale=0.5):
+    """Runs the kernels' forward and backward on seeded inputs -> (device outputs, host inputs); ctr: the one-element device
+    counter added to the dropout seed (as functional.py passes it)."""
+    o = ops()
+    inner = H * dk
+    QKV, QKVr = rnd(B * max(Lq, Lk), 3 * inner, dtype=dtype, seed=1, scale=qk_scale)      # larger scale: more peaked softmax
     q, k, v = QKV[:B * Lq, :inner], QKV[:B * Lk, inner:2 * inner], QKV[:B * Lk, 2 * inner:]
     DO, DOr = rnd(B * Lq, inner, dtype=dtype, seed=2)
     table = 0.5 * torch.randn(32, H, generator=torch.Generator().manual_seed(3))
-    causal = mode == "dec"
     has_bias = mode != "cross"
     lut, rz = o.t5_rel_bucket_lut(Lq, Lk, bidirectional=(mode == "enc"), num_buckets=32, max_distance=128)
-    kw = dict(bias_table=table.cuda() if has_bias else None, lut=lut.cuda() if has_bias else None, rel_zero=rz, causal=causal)
+    kw = dict(bias_table=table.cuda() if has_bias else None, lut=lut.cuda() if has_bias else None, rel_zero=rz, causal=mode == "dec",
+              dropout_p=p, seed=seed, seed_ptr=ctr)
     ctx, lse = o.t5_attention_fwd(q, k, v, B, H, Lq, Lk, dk, **kw)
-    # reference (oracle arithmetic, no projections)
-    qr = QKVr[:B * Lq, :inner].clone().requires_grad_(True)
-    kr = QKVr[:B * Lk, inner:2 * inner].clone().requires_grad_(True)
-    vr = QKVr[:B * Lk, 2 * inner:].clone().requires_grad_(True)
-    tr = table.clone().requires_grad_(True)
-    s = qr.view(B, Lq, H, dk).transpose(1, 2) @ kr.view(B, Lk, H, dk).transpose(1, 2).transpose(-1, -2)
-    if has_bias:
-        s = s + ot5.t5_bias(tr, Lq, Lk, bidirectional=(mode == "enc"), dims=dims)[None]
-    if causal:
-        s = s + torch.where(torch.arange(Lk)[None, :] > torch.arange(Lq)[:, None], torch.finfo(torch.float32).min, 0.0)
-    p = torch.softmax(s, -1)
-    ref = (p @ vr.view(B, Lk, H, dk).transpose(1, 2)).transpose(1, 2).reshape(B * Lq, inner)
-    close(ctx, ref, dtype, "t5 attn fwd")
-    ref.backward(DOr)
     dQKV = torch.zeros_like(QKV)
     dq, dk_, dv = dQKV[:B * Lq, :inner], dQKV[:B * Lk, inner:2 * inner], dQKV[:B * Lk, 2 * inner:]
     dtab = torch.zeros(32, H, device="cuda")
     o.t5_attention_bwd(q, k, v, ctx, DO, lse, dq, dk_, dv, B, H, Lq, Lk, dk, dbias_table=dtab if has_bias else None, **kw)
-    close(dq, qr.grad, dtype, "t5 dq")
-    close(dk_, kr.grad, dtype, "t5 dk")
-    close(dv, vr.grad, dtype, "t5 dv")
-    if has_bias:
-        close(dtab, tr.grad, dtype, "t5 dbias")
+    return (ctx, lse, dq, dk_, dv, dtab if has_bias else None), (QKVr, DOr, table)
+
+
+@pytest.mark.parametrize("dtype", DTYPES)
+@pytest.mark.parametrize("mode,B,H,Lq,Lk,dk,p,multi", _attn_cases(T5_ATTN_SHAPES) + _attn_cases(T5_ATTN_MULTI_SHAPES, multi=True))
+def test_t5_attention(dtype, mode, B, H, Lq, Lk, dk, p, multi, monkeypatch):
+    """Forward (ctx and the un-dropped lse) and backward (dq, dk, dv, bias-table gradient) of every T5 attention kernel path
+    against float64.  With p > 0 the reference multiplies the probabilities by the mask `dropout_apply` draws over a
+    contiguous [B, H, Lq, Lk] tensor of ones (element (b, h, i, j) at ((b*H + h)*Lq + i)*Lk + j, the index every attention
+    kernel hashes), seeded through a device counter."""
+    if multi:
+        monkeypatch.setenv("KLAB_T5_ATTN_MULTI", "1")
+    seed, ctr = 1234, torch.tensor([987654321], dtype=torch.int64, device="cuda")
+    got, (QKVr, DOr, table) = t5_attention_case(dtype, mode, B, H, Lq, Lk, dk, p, seed=seed, ctr=ctr)
+    mask = ops().dropout_apply(torch.ones(B, H, Lq, Lk, device="cuda"), p, seed, ctr).double().cpu() if p > 0 else None
+    ref = t5_attention_reference(QKVr, DOr, table, mode, B, H, Lq, Lk, dk, mask)
+    for name, g, r in zip(("t5 attn fwd", "t5 lse", "t5 dq", "t5 dk", "t5 dv", "t5 dbias"), got, ref):
+        if r is not None:
+            close(g, r, dtype, name)
 
 
 @pytest.mark.parametrize("mode,B,H,Lk,dk,t", [("self", 5, 3, 20, 64, 0), ("self", 5, 3, 20, 64, 7), ("self", 3, 2, 20, 64, 19), ("cross", 4, 12, 96, 64, 0),
